@@ -228,6 +228,39 @@ def run_reference(A, B, threads, max_runs, warmup, budget_s=240.0):
     return info
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, alns):
+    """Writes the alignment records a caller of the timed path receives, so that two builds can be
+    compared record for record on the same seeded pair:
+      fields.npy       (n, 9) float64, columns lib.ALN_FIELDS, in the order the path returns them
+      trace.npy        float32, the trace bytes of all n records concatenated
+      trace_offset.npy (n + 1,) float64, record i's trace is trace[offset[i]:offset[i + 1]]
+      rows.npy         (n,) float64, which records of the step these are
+    Above DUMP_BYTES in all, a fixed seeded sample of the records is written (rows says which)."""
+    n = len(alns)
+    tlen = alns.fields[:, 8].astype(np.int64)
+
+    def nbytes(rows):
+        return len(rows) * (9 * 8 + 8 + 8) + 8 + 4 * int(tlen[rows].sum())
+
+    rows = np.arange(n)
+    k = n
+    while nbytes(rows) > DUMP_BYTES:
+        k = k * 9 // 10
+        rows = np.sort(np.random.default_rng(SEED).permutation(n)[:k])
+    toff = np.concatenate([[0], np.cumsum(tlen[rows])])
+    trace = np.zeros(int(toff[-1]), dtype=np.float32)
+    for j, i in enumerate(rows):
+        trace[toff[j]:toff[j + 1]] = alns.trace(i)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "fields.npy"), alns.fields[rows].astype(np.float64))
+    np.save(os.path.join(out_dir, "trace.npy"), trace)
+    np.save(os.path.join(out_dir, "trace_offset.npy"), toff.astype(np.float64))
+    np.save(os.path.join(out_dir, "rows.npy"), rows.astype(np.float64))
+
+
 def workload_text(per_gpu_bp, n):
     return ("synthetic %d Mbp genome (%d contigs) vs 5%%-diverged copy%s, SV breaks every ~%d kbp, seed %d; "
             "FastGA defaults -f10 -c85 -s1000 -l100 -i.7"
@@ -258,7 +291,11 @@ def run():
     ap.add_argument("--impl", default="b200")
     ap.add_argument("--per-gpu-bp", type=int, default=PER_GPU_BP)
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the alignment records of the last timed step to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -379,7 +416,7 @@ def run():
     else:
         e2e_step = lambda: lib.fastga(pA, pB)
     e2e_step()
-    ms_e2e, outs2 = timed(e2e_step, max(1, min(args.steps, 3)))
+    ms_e2e, outs2 = timed(e2e_step, args.steps)
     st2 = outs2[-1][1]
 
     # gather the per-rank record streams on rank 0 (variable length; the path's only collective)
@@ -396,6 +433,8 @@ def run():
             dist.destroy_process_group()
         return None
 
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, final)
     gpu_md5 = canonical_md5(final.canonical_lines_unsorted())
     steps = args.steps
     # roofline of the seed-merge kernel (the kernel north_star grades): algorithmic bytes on the

@@ -2,6 +2,7 @@
 unmodified reference built into oracle/_ref (binaries + libfastga_ref.so)."""
 import ctypes as C
 import hashlib
+import json
 import os
 import re
 import subprocess
@@ -16,8 +17,31 @@ REF_SO = os.path.join(REF_DIR, "libfastga_ref.so")
 _orc = None
 
 
+GOLDEN = os.path.join(ROOT, "tests", "golden")
+_runs = None
+
+
 def have_ref():
     return os.path.exists(os.path.join(REF_DIR, "FastGA")) and os.path.exists(REF_SO)
+
+
+def reference_run(key):
+    """What the unmodified reference produced for one test input, as stored in
+    tests/golden/reference_runs.json by tests/golden/make_golden.py."""
+    global _runs
+    if _runs is None:
+        with open(os.path.join(GOLDEN, "reference_runs.json")) as f:
+            _runs = json.load(f)
+    return _runs[key]
+
+
+def reference_paths(key):
+    """The reference's Local_Alignment results for one list of calls (tests/golden/reference_paths.npz):
+    (n, 6) int32 rows abpos bbpos aepos bepos diffs tlen, and the traces of all calls concatenated."""
+    with np.load(os.path.join(GOLDEN, "reference_paths.npz")) as z:
+        paths, traces = z[key + "_paths"], z[key + "_traces"]
+    toff = np.concatenate([[0], np.cumsum(paths[:, 5].astype(np.int64))])
+    return paths, [traces[toff[i]:toff[i + 1]] for i in range(len(paths))]
 
 
 def orc():
@@ -153,6 +177,11 @@ def oneview_records(path):
     sorted (SURVEY 8c)."""
     out = subprocess.run([os.path.join(REF_DIR, "ONEview"), path], stdout=subprocess.PIPE, text=True,
                          check=True).stdout
+    return records_from_text(out)
+
+
+def records_from_text(out):
+    """canonical records of ONEcode ASCII text: ONEview's dump, or an ASCII .1aln as it is"""
     recs, cur = [], None
     for line in out.split("\n"):
         if line.startswith("A "):

@@ -1,7 +1,6 @@
 """-m gpu: the align.h seam -- fgb_local_alignments (batched Local_Alignment) against the UNMODIFIED
-reference's Local_Alignment (oracle/_ref/libfastga_ref.so) on random call tuples, borders included."""
-import ctypes as C
-
+reference's Local_Alignment on random call tuples, borders included (its results are stored in
+tests/golden/reference_paths.npz by tests/golden/make_golden.py)."""
 import numpy as np
 import pytest
 
@@ -11,19 +10,9 @@ from fastga_b200 import formats, lib, synth
 pytestmark = pytest.mark.gpu
 
 
-class Path(C.Structure):
-    _fields_ = [("trace", C.c_void_p), ("tlen", C.c_int), ("diffs", C.c_int), ("abpos", C.c_int),
-                ("bbpos", C.c_int), ("aepos", C.c_int), ("bepos", C.c_int)]
-
-
-class Alignment(C.Structure):
-    _fields_ = [("path", C.POINTER(Path)), ("flags", C.c_uint32), ("aseq", C.c_void_p), ("bseq", C.c_void_p),
-                ("alen", C.c_int), ("blen", C.c_int)]
-
-
-@pytest.mark.skipif(not ol.have_ref(), reason="oracle/_ref not built")
-@pytest.mark.parametrize("borders", [False, True])
-def test_batched_local_alignment_matches_reference(borders):
+def seam_jobs(borders):
+    """six contigs, their diverged copies and 300 random Local_Alignment call tuples on them:
+    (A, B, jobs (i, j, comp, low, hgh, anti, lbord, hbord))"""
     rng = np.random.default_rng(41 + int(borders))
     ncont = 6
     A = [rng.integers(0, 4, int(rng.integers(3000, 40000)), dtype=np.uint8) for _ in range(ncont)]
@@ -33,8 +22,6 @@ def test_batched_local_alignment_matches_reference(borders):
         b = synth.diverged_copy(rng, a, rate, sv_every=0, inversions=False)      # small mutations only
         pad.append(int(rng.integers(0, 300)))
         B.append(np.concatenate([rng.integers(0, 4, pad[-1], dtype=np.uint8), b]))
-    gA, gB = formats.genome_from_arrays(A), formats.genome_from_arrays(B)
-    dA, dB = lib.DeviceGenome(gA, want_revcomp=True), lib.DeviceGenome(gB)
     jobs = []
     for _ in range(300):
         i = int(rng.integers(0, ncont))
@@ -51,30 +38,24 @@ def test_batched_local_alignment_matches_reference(borders):
             lbd = int(rng.integers(0, 40)) if rng.random() < 0.7 else -1
             hbd = int(rng.integers(0, 40)) if rng.random() < 0.7 else -1
         jobs.append((i, i, comp, low, hgh, anti, lbd, hbd))
-    jobs = np.array(jobs, dtype=np.int32)
+    return A, B, np.array(jobs, dtype=np.int32)
+
+
+@pytest.mark.parametrize("borders", [False, True])
+def test_batched_local_alignment_matches_reference(borders):
+    A, B, jobs = seam_jobs(borders)
+    gA, gB = formats.genome_from_arrays(A), formats.genome_from_arrays(B)
+    dA, dB = lib.DeviceGenome(gA, want_revcomp=True), lib.DeviceGenome(gB)
     paths, toff, traces = lib.local_alignments(dA, dB, jobs, gA.freq)
 
-    ref = C.CDLL(ol.REF_SO)
-    ref.New_Work_Data.restype = C.c_void_p
-    ref.New_Align_Spec.restype = C.c_void_p
-    ref.New_Align_Spec.argtypes = [C.c_double, C.c_int, C.POINTER(C.c_float), C.c_int]
-    ref.Local_Alignment.argtypes = [C.POINTER(Alignment), C.c_void_p, C.c_void_p] + [C.c_int] * 5
-    freq = (C.c_float * 4)(*[float(v) for v in gA.freq])
-    work = ref.New_Work_Data()
-    spec = ref.New_Align_Spec(0.7, 100, freq, 0)
-    fA = [ol._framed(a) for a in A]
-    fAC = [ol._framed(3 - a[::-1]) for a in A]
-    fB = [ol._framed(b) for b in B]
+    want, wtrace = ol.reference_paths("seam_%s" % borders)
+    assert len(want) == len(jobs)
     nonempty = 0
-    for q, (i, j, comp, low, hgh, anti, lbd, hbd) in enumerate(jobs.tolist()):
-        a, b = (fAC[i] if comp else fA[i]), fB[j]
-        p = Path()
-        al = Alignment(C.pointer(p), 2 if comp else 0, a.ctypes.data + 1, b.ctypes.data + 1, len(a) - 2, len(b) - 2)
-        assert ref.Local_Alignment(C.byref(al), work, spec, low, hgh, anti, lbd, hbd) == 0
-        rt = np.ctypeslib.as_array(C.cast(p.trace, C.POINTER(C.c_uint16)), shape=(max(p.tlen, 1),))[:p.tlen]
+    for q in range(len(jobs)):
         got = paths[q]
         assert got[6] == 0, (q, got)
-        assert (p.abpos, p.bbpos, p.aepos, p.bepos, p.diffs, p.tlen) == tuple(int(v) for v in got[:6]), (q, jobs[q])
-        assert np.array_equal(rt.astype(np.uint8), traces[int(toff[q]):int(toff[q]) + p.tlen]), q
-        nonempty += int(p.aepos > p.abpos)
+        assert tuple(int(v) for v in want[q]) == tuple(int(v) for v in got[:6]), (q, jobs[q])
+        tlen = int(want[q][5])
+        assert np.array_equal(wtrace[q], traces[int(toff[q]):int(toff[q]) + tlen]), q
+        nonempty += int(want[q][2] > want[q][0])
     assert nonempty > 100

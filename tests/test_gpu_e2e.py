@@ -1,5 +1,7 @@
-"""-m gpu: the reference-facing call (fgb_fastga, host buffers) against the UNMODIFIED reference run
-on the same box (oracle/_ref/FastGA), records compared bit-exactly after the canonical sort."""
+"""-m gpu: the reference-facing call (fgb_fastga, host buffers) against runs of the UNMODIFIED
+reference on the same inputs (stored by tests/golden/make_golden.py), records compared bit-exactly
+after the canonical sort."""
+import hashlib
 import os
 import tempfile
 
@@ -12,46 +14,48 @@ from fastga_b200 import formats, lib, synth
 pytestmark = pytest.mark.gpu
 
 
-def _vs_reference(seed, total, ncontig, div, sv, threads=8, per_scaffold=1):
+E2E_PAIRS = {"small_pair": (11, 1_200_000, 3, 0.05, 60_000, 1),
+             "scaffolded_15pct": (12, 2_000_000, 6, 0.15, 40_000, 3),
+             # no SV breaks: contig-long alignments -> pebble arenas overflow and the retry path runs
+             "long_alignments": (13, 6_000_000, 3, 0.03, 0, 1),
+             "10mbp": (14, 10_000_000, 5, 0.05, 200_000, 1)}
+
+
+def _vs_reference(name):
+    seed, total, ncontig, div, sv, per_scaffold = E2E_PAIRS[name]
     A, B = synth.make_pair(seed, total, ncontig, div, sv_every=sv)
     with tempfile.TemporaryDirectory() as wd:
         formats.write_fasta(os.path.join(wd, "A.fasta"), synth.scaffolds_of(A, "sa", per_scaffold))
         formats.write_fasta(os.path.join(wd, "B.fasta"), synth.scaffolds_of(B, "sb", per_scaffold))
-        log = ol.ref_fastga(wd, "A", "B", threads=threads)
-        st = ol.parse_fastga_log(log)
-        ref = ol.oneview_records(os.path.join(wd, "ref.1aln"))
         gA = formats.genome_from_fasta(os.path.join(wd, "A.fasta"))
         gB = formats.genome_from_fasta(os.path.join(wd, "B.fasta"))
-        assert np.array_equal(np.fromfile(os.path.join(wd, ".A.bps"), dtype=np.uint8), gA.bps)
+    ref = ol.reference_run("e2e/" + name)
+    st = ref["counters"]
+    assert hashlib.md5(gA.bps.tobytes()).hexdigest() == ref["bps_md5_A"]      # the .bps FAtoGDB wrote
     alns, stats = lib.fastga(gA, gB)
     assert stats["nseeds"] == st["seeds"]
     assert stats["nhits"] == st["hits"]
     assert alns.nraw == st["alns"]
-    assert len(alns) == st["kept"]
+    assert len(alns) == st["kept"] == ref["records"]
     mine = alns.canonical_lines()
-    assert ol.md5_lines(mine) == ol.md5_lines(ref)
+    assert ol.md5_lines(mine) == ref["aln_md5"]
     return stats
 
 
-@pytest.mark.skipif(not ol.have_ref(), reason="oracle/_ref not built")
 def test_small_pair_bit_exact_vs_reference():
-    _vs_reference(11, 1_200_000, 3, 0.05, 60_000)
+    _vs_reference("small_pair")
 
 
-@pytest.mark.skipif(not ol.have_ref(), reason="oracle/_ref not built")
 def test_scaffolded_15pct_bit_exact_vs_reference():
-    _vs_reference(12, 2_000_000, 6, 0.15, 40_000, per_scaffold=3)
+    _vs_reference("scaffolded_15pct")
 
 
-@pytest.mark.skipif(not ol.have_ref(), reason="oracle/_ref not built")
 def test_long_alignments_exercise_arena_retry():
-    # no SV breaks: contig-long alignments -> pebble arenas overflow and the retry path runs
-    _vs_reference(13, 6_000_000, 3, 0.03, 0)
+    _vs_reference("long_alignments")
 
 
-@pytest.mark.skipif(not ol.have_ref(), reason="oracle/_ref not built")
 def test_10mbp_bit_exact_vs_reference():
-    _vs_reference(14, 10_000_000, 5, 0.05, 200_000)
+    _vs_reference("10mbp")
 
 
 @pytest.mark.parametrize("gap", ["0", "3000", "1000000000"])
@@ -112,39 +116,45 @@ def test_example_regions_wide_band_chunks_bit_exact_vs_oracle():
     assert alns.canonical_lines() == want["lines"]
 
 
-@pytest.mark.skipif(not ol.have_ref(), reason="oracle/_ref not built")
+def gix_genome():
+    A, _ = synth.make_pair(17, 2_500_000, 5, 0.05, sv_every=100_000)
+    return A
+
+
 def test_gix_files_match_reference_gixmake():
     """SURVEY 8 a-4: the .ktab entry stream, the stub index and the part split produced from the
-    device table equal what the reference GIXmake writes (equal k-mers canonicalised), and the
-    reference's own GIX files import back into the identical device table."""
-    A, _ = synth.make_pair(17, 2_500_000, 5, 0.05, sv_every=100_000)
-    with tempfile.TemporaryDirectory() as wd:
-        formats.write_fasta(os.path.join(wd, "A.fasta"), synth.scaffolds_of(A, "sa", 2))
-        ol.run_ref(["GIXmake", "-T4", "-P" + wd, "A"], cwd=wd)
-        ref = formats.read_gix(os.path.join(wd, "A.gix"))
+    device table equal what the reference GIXmake writes (equal k-mers canonicalised; stored by
+    tests/golden/make_golden.py), and that entry stream imports back into the identical device table."""
+    A = gix_genome()
+    ref = ol.reference_run("gix/gixmake")
     g = formats.genome_from_arrays(A)
     dg = lib.DeviceGenome(g)
     gx = lib.DeviceGix.build(dg)
     tab, pstart, buck = gx.download()
-    assert gx.n == ref.n
+    assert gx.n == ref["n"]
     pb, cb = formats.gix_bytes(g)
-    assert (pb, cb) == (ref.post_bytes, ref.cont_bytes) == (gx.post_bytes, max(gx.cont_bytes, cb))
-    assert np.array_equal(pstart[1:].astype(np.int64), ref.index)
-    assert np.array_equal(dg.perm, ref.perm[:g.ncontig])
+    assert (pb, cb) == (ref["post_bytes"], ref["cont_bytes"]) == (gx.post_bytes, max(gx.cont_bytes, cb))
+    index = pstart[1:].astype(np.int64)
+    assert hashlib.md5(index.tobytes()).hexdigest() == ref["index_md5"]
+    assert list(dg.perm) == ref["perm"][:g.ncontig]
     # part split from the sampler histogram (GIXmake.c:655-691)
     nparts = formats.gix_nparts(g.seqtot, max(g.ncontig, 4), pb, cb, nthreads=4)
-    assert nparts == ref.nparts
+    assert nparts == ref["nparts"]
     ks = formats.ksplit_from_buckets(buck, nparts)
     part_first = np.array([int(pstart[k << 14]) for k in ks[:-1]], dtype=np.int64)
     part_n = np.diff(np.concatenate([part_first, [gx.n]]))
-    assert list(part_n) == ref.part_n
+    assert list(part_n) == ref["part_n"]
     ent = gx.export_ktab(part_first) if gx.cont_bytes == cb else None
     if ent is None:     # device handle counts real contigs only; re-encode with the padded width
         ent = formats.ktab_entries_from_table(tab, pb, cb, part_first)
-    E = ref.esize
-    assert np.array_equal(formats.canonical_ktab(ent, E, ref.index), formats.canonical_ktab(ref.entries, E, ref.index))
-    # and the reverse direction: reference files -> device table
-    imp = lib.DeviceGix.import_ktab(ref)
+    E = 9 + pb + cb
+    canon = formats.canonical_ktab(ent, E, index)
+    assert hashlib.md5(canon.tobytes()).hexdigest() == ref["entries_md5"]
+    # and the reverse direction: the reference's entries (canonical form: the order of equal k-mers
+    # differs from the device table's) -> device table
+    f = formats.GixFile()
+    f.entries, f.n, f.post_bytes, f.cont_bytes, f.index, f.ncontig = canon, gx.n, pb, cb, index, len(ref["perm"])
+    imp = lib.DeviceGix.import_ktab(f)
     itab, ipstart, _ = imp.download()
     assert np.array_equal(ipstart, pstart)
     key = lambda t: np.lexsort((t[:, 0] & np.uint64(0xffffffffffff), t[:, 0] >> np.uint64(48), t[:, 1]))
@@ -152,22 +162,19 @@ def test_gix_files_match_reference_gixmake():
 
 
 # ---------------------------------------------------------------------------------------------
-#  edge cases (tests/edge_cases.py): ragged / degenerate inputs, against the reference
+#  edge cases (tests/edge_cases.py): ragged / degenerate inputs, against the reference's runs on
+#  them (tests/golden/reference_runs.json)
 # ---------------------------------------------------------------------------------------------
 
 import edge_cases  # noqa: E402
 
 
-@pytest.mark.skipif(not ol.have_ref(), reason="oracle/_ref not built")
 @pytest.mark.parametrize("name", sorted(edge_cases.CASES))
 def test_edge_case_bit_exact_vs_reference(name):
     A, B, threads, check = edge_cases.CASES[name]()
-    with tempfile.TemporaryDirectory() as wd:
-        formats.write_fasta(os.path.join(wd, "A.fasta"), synth.scaffolds_of(A, "sa", 1))
-        formats.write_fasta(os.path.join(wd, "B.fasta"), synth.scaffolds_of(B, "sb", 1))
-        st = ol.parse_fastga_log(ol.ref_fastga(wd, "A", "B", threads=threads))
-        ref = ol.oneview_records(os.path.join(wd, "ref.1aln"))
+    ref = ol.reference_run("edge/" + name)
     alns, stats = lib.fastga(formats.genome_from_arrays(A), formats.genome_from_arrays(B))
-    assert stats["nseeds"] == st.get("seeds", 0)
-    assert alns.canonical_lines() == ref
+    assert stats["nseeds"] == ref["counters"].get("seeds", 0)
+    lines = alns.canonical_lines()
+    assert len(lines) == ref["records"] and ol.md5_lines(lines) == ref["aln_md5"]
     check(alns, stats["nhits"])

@@ -237,22 +237,27 @@ def test_extend_matches_oracle(small_pair):
 
 
 # ---------------------------------------------------------------------------------------------
-#  the reference's extern sort seams (msd_sort / rmsd_sort) against libfastga_ref.so
+#  the reference's extern sort seams (msd_sort / rmsd_sort) against what libfastga_ref.so returned
+#  on the same inputs (tests/golden/reference_runs.json)
 # ---------------------------------------------------------------------------------------------
 
 import ctypes as C
+import hashlib
 
 
 class _Range(C.Structure):
     _fields_ = [("beg", C.c_int), ("end", C.c_int), ("off", C.c_int64)]
 
 
-@pytest.mark.skipif(not ol.have_ref(), reason="oracle/_ref not built")
-def test_msd_sort_seam_matches_reference():
-    from fastga_b200 import load_library
-    L, ref = load_library(), C.CDLL(ol.REF_SO)
+MSD_ARGTYPES = [C.c_void_p, C.c_int64, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_int]
+RMSD_ARGTYPES = [C.c_void_p, C.c_int64, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_void_p]
+
+
+def msd_input():
+    """records in GIXmake's shape on EXAMPLE (swide 15, KBYTES 10): (array + 16 pad bytes, n, rsize,
+    ksize, part, beg, end)"""
     rng = np.random.default_rng(9)
-    rsize, ksize, beg, end = 15, 10, 3, 40           # GIXmake's shape on EXAMPLE: swide 15, KBYTES 10
+    rsize, ksize, beg, end = 15, 10, 3, 40
     counts = rng.integers(0, 3000, end - beg)
     counts[5] = 0
     n = int(counts.sum())
@@ -261,45 +266,53 @@ def test_msd_sort_seam_matches_reference():
     arr[:, 3:9] &= 0x03                              # few distinct keys -> long equal runs and LCPs
     part = np.zeros(1024, dtype=np.int64)
     part[beg:end] = counts * rsize
-    a1 = np.concatenate([arr.reshape(-1), np.zeros(16, np.uint8)])
-    a2 = a1.copy()
-    argt = [C.c_void_p, C.c_int64, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_int]
-    ref.msd_sort.argtypes = argt
-    L.fgb_msd_sort.argtypes = argt
-    ref.msd_sort(a1.ctypes.data, n, rsize, ksize, part.ctypes.data, beg, end, 4)
-    L.fgb_msd_sort(a2.ctypes.data, n, rsize, ksize, part.ctypes.data, beg, end, 4)
-    r1, r2 = a1[:n * rsize].reshape(n, rsize), a2[:n * rsize].reshape(n, rsize)
-    assert a1[n * rsize] == a2[n * rsize] == 1
-    assert np.array_equal(r1[:, :ksize], r2[:, :ksize])          # LCP byte + key bytes identical
-    run = np.cumsum(r1[:, 0] != 0)                               # payloads: same multiset per equal-key run
-    def canon(r):
-        pay = np.zeros(n, dtype=np.uint64)
-        for k in range(ksize, rsize):
-            pay |= r[:, k].astype(np.uint64) << np.uint64(8 * (k - ksize))
-        return pay[np.lexsort((pay, run))]
-    assert np.array_equal(canon(r1), canon(r2))
+    return np.concatenate([arr.reshape(-1), np.zeros(16, np.uint8)]), n, rsize, ksize, part, beg, end
 
 
-@pytest.mark.skipif(not ol.have_ref(), reason="oracle/_ref not built")
-def test_rmsd_sort_seam_matches_reference():
+def msd_payload_md5(r, ksize):
+    """payloads of the sorted records with every equal-key run put in order (the sort is not stable)"""
+    n, rsize = r.shape
+    run = np.cumsum(r[:, 0] != 0)
+    pay = np.zeros(n, dtype=np.uint64)
+    for k in range(ksize, rsize):
+        pay |= r[:, k].astype(np.uint64) << np.uint64(8 * (k - ksize))
+    return hashlib.md5(pay[np.lexsort((pay, run))].tobytes()).hexdigest()
+
+
+def test_msd_sort_seam_matches_reference():
     from fastga_b200 import load_library
-    L, ref = load_library(), C.CDLL(ol.REF_SO)
+    L = load_library()
+    a, n, rsize, ksize, part, beg, end = msd_input()
+    L.fgb_msd_sort.argtypes = MSD_ARGTYPES
+    L.fgb_msd_sort(a.ctypes.data, n, rsize, ksize, part.ctypes.data, beg, end, 4)
+    want = ol.reference_run("seam/msd_sort")
+    r = a[:n * rsize].reshape(n, rsize)
+    assert a[n * rsize] == want["sentinel"] == 1
+    # LCP byte + key bytes identical, payloads the same multiset per equal-key run
+    assert hashlib.md5(np.ascontiguousarray(r[:, :ksize]).tobytes()).hexdigest() == want["keys_md5"]
+    assert msd_payload_md5(r, ksize) == want["payload_md5"]
+
+
+def rmsd_input():
+    """FastGA's seed record on EXAMPLE (swide 9): (array, n, rsize, nparts, part, nthreads)"""
     rng = np.random.default_rng(10)
-    rsize, nparts, nthreads = 9, 37, 8                # FastGA's seed record on EXAMPLE: swide 9
+    rsize, nparts, nthreads = 9, 37, 8
     counts = rng.integers(0, 5000, nparts)
     counts[[0, 7]] = 0
     n = int(counts.sum())
     arr = rng.integers(0, 256, (n, rsize), dtype=np.uint8)
     arr[:, 5:] &= 0x07
     part = (counts * rsize).astype(np.int64)
-    a1, a2 = arr.reshape(-1).copy(), arr.reshape(-1).copy()
-    p1, p2 = (_Range * nthreads)(), (_Range * nthreads)()
-    argt = [C.c_void_p, C.c_int64, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_void_p]
-    ref.rmsd_sort.argtypes = argt
-    L.fgb_rmsd_sort.argtypes = argt
-    n1 = ref.rmsd_sort(a1.ctypes.data, n, rsize, rsize, nparts, part.ctypes.data, nthreads, p1)
-    n2 = L.fgb_rmsd_sort(a2.ctypes.data, n, rsize, rsize, nparts, part.ctypes.data, nthreads, p2)
-    assert n1 == n2
-    assert [(p1[i].beg, p1[i].end, p1[i].off) for i in range(n1)] == \
-           [(p2[i].beg, p2[i].end, p2[i].off) for i in range(n2)]
-    assert np.array_equal(a1, a2)
+    return arr.reshape(-1).copy(), n, rsize, nparts, part, nthreads
+
+
+def test_rmsd_sort_seam_matches_reference():
+    from fastga_b200 import load_library
+    L = load_library()
+    a, n, rsize, nparts, part, nthreads = rmsd_input()
+    p = (_Range * nthreads)()
+    L.fgb_rmsd_sort.argtypes = RMSD_ARGTYPES
+    n2 = L.fgb_rmsd_sort(a.ctypes.data, n, rsize, rsize, nparts, part.ctypes.data, nthreads, p)
+    want = ol.reference_run("seam/rmsd_sort")
+    assert [[p[i].beg, p[i].end, p[i].off] for i in range(n2)] == want["ranges"]
+    assert hashlib.md5(a.tobytes()).hexdigest() == want["md5"]

@@ -1,8 +1,7 @@
 """-m gpu: trace points -> edit scripts (fgb_compute_trace_pts, SURVEY row a-17) against the
-UNMODIFIED reference's Compute_Trace_PTS (oracle/_ref/libfastga_ref.so) on the alignments the path
-itself emits: same int script, same diffs, for every record."""
-import ctypes as C
-import os
+UNMODIFIED reference's Compute_Trace_PTS on the alignments the path itself emits: same int script,
+same diffs, for every record (the reference's scripts are stored by tests/golden/make_golden.py)."""
+import hashlib
 
 import numpy as np
 import pytest
@@ -13,68 +12,46 @@ from fastga_b200 import formats, lib, synth
 pytestmark = pytest.mark.gpu
 
 
-class Path(C.Structure):
-    _fields_ = [("trace", C.c_void_p), ("tlen", C.c_int), ("diffs", C.c_int), ("abpos", C.c_int),
-                ("bbpos", C.c_int), ("aepos", C.c_int), ("bepos", C.c_int)]
-
-
-class Alignment(C.Structure):
-    _fields_ = [("path", C.POINTER(Path)), ("flags", C.c_uint32), ("aseq", C.c_void_p), ("bseq", C.c_void_p),
-                ("alen", C.c_int), ("blen", C.c_int)]
-
-
-def _reference_scripts(gA, gB, alns, limit=None):
-    """Compute_Trace_PTS(aln, work, 100, GREEDIEST, 1, -1) as ALNtoPAF.c:251-272 calls it"""
-    ref = C.CDLL(ol.REF_SO)
-    ref.New_Work_Data.restype = C.c_void_p
-    ref.Compute_Trace_PTS.argtypes = [C.POINTER(Alignment), C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int]
-    work = ref.New_Work_Data()
-    A = [ol._framed(gA.contig(c)) for c in range(gA.ncontig)]
-    B = [ol._framed(gB.contig(c)) for c in range(gB.ncontig)]
-    BC = [ol._framed(3 - gB.contig(c)[::-1]) for c in range(gB.ncontig)]
-    out = []
-    n = len(alns) if limit is None else min(limit, len(alns))
-    for i in range(n):
-        comp, ar, br, ab, bb, ae, be, df, tl = (int(x) for x in alns.fields[i])
-        pts = alns.trace(i).astype(np.uint16)            # Decompress_TraceTo16
-        p = Path(pts.ctypes.data, tl, df, ab, bb, ae, be)
-        a, b = A[ar], (BC[br] if comp else B[br])
-        al = Alignment(C.pointer(p), 2 if comp else 0, a.ctypes.data + 1, b.ctypes.data + 1, len(a) - 2, len(b) - 2)
-        assert ref.Compute_Trace_PTS(C.byref(al), work, 100, 0, 1, -1) == 0
-        sc = np.ctypeslib.as_array(C.cast(p.trace, C.POINTER(C.c_int32)), shape=(max(p.tlen, 1),))[:p.tlen].copy()
-        out.append((sc, p.diffs))
-    return out
-
-
-def _check_pair(seed, total, ncontig, div, sv, flip=()):
+def trace_pair(seed, total, ncontig, div, sv, flip=()):
     A, B = synth.make_pair(seed, total, ncontig, div, sv_every=sv)
     for i in flip:                                   # whole contigs on the opposite strand
         B[i] = (3 - B[i][::-1]).astype(np.uint8)
-    gA, gB = formats.genome_from_arrays(A), formats.genome_from_arrays(B)
+    return formats.genome_from_arrays(A), formats.genome_from_arrays(B)
+
+
+TRACE_PAIRS = {"5pct": (21, 3_000_000, 4, 0.05, 60_000), "15pct_both_strands": (22, 2_000_000, 5, 0.15, 30_000, (0, 3))}
+
+
+def _check_pair(name):
+    """the reference's Compute_Trace_PTS(aln, work, 100, GREEDIEST, 1, -1), as ALNtoPAF.c:251-272
+    calls it, on the same alignments: per record its diffs, script length and script md5
+    (tests/golden/reference_runs.json)"""
+    gA, gB = trace_pair(*TRACE_PAIRS[name])
     alns, _ = lib.fastga(gA, gB)
     assert len(alns) > 0
     dA, dB = lib.DeviceGenome(gA), lib.DeviceGenome(gB, want_revcomp=True)
     soff, script, diffs = lib.compute_trace_pts(dA, dB, alns)
-    want = _reference_scripts(gA, gB, alns)
+    want = {tuple(r[:7]): r[7:] for r in ol.reference_run("trace/" + name)["scripts"]}
+    assert len(want) == len(alns)
     assert (diffs >= 0).all()
     ncomp = 0
-    for i, (sc, df) in enumerate(want):
-        got = script[soff[i]:soff[i + 1]]
+    for i in range(len(alns)):
+        key = tuple(int(x) for x in alns.fields[i, :7])
+        df, slen, md5 = want[key]
+        got = np.ascontiguousarray(script[soff[i]:soff[i + 1]], dtype=np.int32)
         assert df == diffs[i], (i, df, int(diffs[i]))
-        assert np.array_equal(got, sc), (i, got[:8], sc[:8])
+        assert len(got) == slen and hashlib.md5(got.tobytes()).hexdigest() == md5, (i, got[:8])
         ncomp += int(alns.fields[i, 0])
-    return len(want), ncomp
+    return len(alns), ncomp
 
 
-@pytest.mark.skipif(not ol.have_ref(), reason="oracle/_ref not built")
 def test_scripts_match_reference_5pct():
-    n, ncomp = _check_pair(21, 3_000_000, 4, 0.05, 60_000)
+    n, ncomp = _check_pair("5pct")
     assert n > 10
 
 
-@pytest.mark.skipif(not ol.have_ref(), reason="oracle/_ref not built")
 def test_scripts_match_reference_15pct_both_strands():
-    n, ncomp = _check_pair(22, 2_000_000, 5, 0.15, 30_000, flip=(0, 3))
+    n, ncomp = _check_pair("15pct_both_strands")
     assert n > 10 and ncomp > 0
 
 

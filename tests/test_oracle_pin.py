@@ -1,8 +1,7 @@
-"""CPU tests that pin the oracle (oracle/fastga_oracle.c) to the UNMODIFIED reference:
-  * committed golden vectors (tests/golden/reference_golden.json, made by tests/golden/make_golden.py
-    from runs of oracle/_ref) -- work without the reference;
-  * live comparisons against oracle/_ref (libfastga_ref.so Local_Alignment, FastGA binaries) when
-    that directory has been built (skipped otherwise)."""
+"""CPU tests that pin the oracle (oracle/fastga_oracle.c) to the UNMODIFIED reference through
+committed golden vectors (tests/golden/reference_golden.json, reference_runs.json and
+reference_paths.npz, made by tests/golden/make_golden.py from runs of oracle/_ref): the reference's
+counters, its alignment records and its Local_Alignment results on the same seeded inputs."""
 import ctypes as C
 import hashlib
 import json
@@ -50,18 +49,8 @@ def test_oracle_reproduces_reference_golden(name):
 
 
 # ---------------------------------------------------------------------------------------------
-#  live pins against oracle/_ref
+#  pins against stored results of oracle/_ref
 # ---------------------------------------------------------------------------------------------
-
-class Path(C.Structure):
-    _fields_ = [("trace", C.c_void_p), ("tlen", C.c_int), ("diffs", C.c_int), ("abpos", C.c_int),
-                ("bbpos", C.c_int), ("aepos", C.c_int), ("bepos", C.c_int)]
-
-
-class Alignment(C.Structure):
-    _fields_ = [("path", C.POINTER(Path)), ("flags", C.c_uint32), ("aseq", C.c_void_p), ("bseq", C.c_void_p),
-                ("alen", C.c_int), ("blen", C.c_int)]
-
 
 class OPath(C.Structure):
     _fields_ = [("abpos", C.c_int), ("bbpos", C.c_int), ("aepos", C.c_int), ("bepos", C.c_int),
@@ -88,13 +77,11 @@ def _mutate(rng, a, rate):
     return np.array(out, dtype=np.int8)
 
 
-@pytest.mark.skipif(not ol.have_ref(), reason="oracle/_ref not built")
 @pytest.mark.parametrize("seed", [1, 2, 3])
 def test_local_alignment_bit_exact_vs_reference_library(seed):
     _la_compare(seed, borders=False)
 
 
-@pytest.mark.skipif(not ol.have_ref(), reason="oracle/_ref not built")
 @pytest.mark.parametrize("seed", [11, 12])
 def test_local_alignment_with_band_borders_vs_reference_library(seed):
     """lbord / hbord >= 0 confine the band to [low-lbord, hgh+hbord] (align.c:1466-1481): what
@@ -103,22 +90,10 @@ def test_local_alignment_with_band_borders_vs_reference_library(seed):
     _la_compare(seed, borders=True)
 
 
-def _la_compare(seed, borders):
-    ref = C.CDLL(ol.REF_SO)
-    orc = ol.orc()
-    ref.New_Work_Data.restype = C.c_void_p
-    ref.New_Align_Spec.restype = C.c_void_p
-    ref.New_Align_Spec.argtypes = [C.c_double, C.c_int, C.POINTER(C.c_float), C.c_int]
-    ref.Local_Alignment.argtypes = [C.POINTER(Alignment), C.c_void_p, C.c_void_p] + [C.c_int] * 5
-    orc.orc_local_alignment.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int] + \
-        [C.c_int] * 6 + [C.POINTER(OPath)]
-    freq = (C.c_float * 4)(.25, .25, .25, .25)
-    work = ref.New_Work_Data()
-    spec = ref.New_Align_Spec(0.7, 100, freq, 0)
-    ospec, _tabs, _ = ol.make_spec(np.array([.25] * 4, np.float32), 0.7)
-    owork = C.c_void_p(orc.orc_new_work())
+def la_calls(seed, borders):
+    """400 Local_Alignment calls on random sequence pairs: (a, b, acomp, low, hgh, anti, lbord, hbord)"""
     rng = np.random.default_rng(seed)
-    for it in range(400):
+    for _ in range(400):
         L = int(rng.integers(300, 5000))
         rate = float(rng.choice([0.0, 0.02, 0.05, 0.1, 0.15, 0.3]))
         core = rng.integers(0, 4, L).astype(np.int8)
@@ -130,7 +105,6 @@ def _la_compare(seed, borders):
         a = np.concatenate([fa, core, ta])
         b = np.concatenate([fb, _mutate(rng, core, rate), tb])
         acomp = int(rng.random() < 0.5)
-        ab, bb = ol._framed(a), ol._framed(b)
         xa, xb = len(fa) + L // 2, len(fb) + L // 2
         d, anti = xa - xb, xa + xb + int(rng.integers(-100, 100))
         low, hgh = d - int(rng.integers(0, 80)), d + int(rng.integers(0, 80))
@@ -138,52 +112,68 @@ def _la_compare(seed, borders):
         if borders:
             lb = int(rng.integers(0, 40)) if rng.random() < 0.7 else -1
             hb = int(rng.integers(0, 40)) if rng.random() < 0.7 else -1
-        p = Path()
-        al = Alignment(C.pointer(p), 2 if acomp else 0, ab.ctypes.data + 1, bb.ctypes.data + 1, len(a), len(b))
-        assert ref.Local_Alignment(C.byref(al), work, spec, low, hgh, anti, lb, hb) == 0
-        rt = np.ctypeslib.as_array(C.cast(p.trace, C.POINTER(C.c_uint16)), shape=(max(p.tlen, 1),))[:p.tlen]
-        rt = rt.astype(np.uint8)
+        yield a, b, acomp, low, hgh, anti, lb, hb
+
+
+def _la_compare(seed, borders):
+    """the oracle's Local_Alignment against the reference's on the calls of la_calls"""
+    orc = ol.orc()
+    orc.orc_local_alignment.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int] + \
+        [C.c_int] * 6 + [C.POINTER(OPath)]
+    ospec, _tabs, _ = ol.make_spec(np.array([.25] * 4, np.float32), 0.7)
+    owork = C.c_void_p(orc.orc_new_work())
+    want, wtrace = ol.reference_paths("la_%s%d" % ("b" if borders else "", seed))
+    for it, (a, b, acomp, low, hgh, anti, lb, hb) in enumerate(la_calls(seed, borders)):
+        ab, bb = ol._framed(a), ol._framed(b)
         op = OPath()
         orc.orc_local_alignment(owork, C.byref(ospec), ab.ctypes.data + 1, len(a), bb.ctypes.data + 1, len(b),
                                 acomp, low, hgh, anti, lb, hb, C.byref(op))
         ot = np.ctypeslib.as_array(op.trace, shape=(max(op.tlen, 1),))[:op.tlen] if op.tlen else np.zeros(0, np.uint8)
-        assert (p.abpos, p.bbpos, p.aepos, p.bepos, p.diffs, p.tlen) == \
-               (op.abpos, op.bbpos, op.aepos, op.bepos, op.diffs, op.tlen), (it, L, rate, acomp, lb, hb)
-        assert np.array_equal(rt, ot), (it, L, rate, acomp, lb, hb)
+        assert tuple(int(v) for v in want[it]) == \
+               (op.abpos, op.bbpos, op.aepos, op.bepos, op.diffs, op.tlen), (it, len(a), acomp, lb, hb)
+        assert np.array_equal(wtrace[it], ot), (it, len(a), acomp, lb, hb)
+    assert it + 1 == len(want)
 
 
-@pytest.mark.skipif(not ol.have_ref(), reason="oracle/_ref not built")
 def test_oracle_vs_live_reference_run(tmp_path):
+    """the oracle against a reference run on a scaffolded pair (tests/golden/reference_runs.json),
+    and the product's FASTA reader against the contig split of the reference's FAtoGDB"""
     A, B = synth.make_pair(31, 600_000, 3, 0.07, sv_every=30_000)
     wd = str(tmp_path)
     formats.write_fasta(os.path.join(wd, "A.fasta"), synth.scaffolds_of(A, "sa", 1))
     formats.write_fasta(os.path.join(wd, "B.fasta"), synth.scaffolds_of(B, "sb", 3))
-    st = ol.parse_fastga_log(ol.ref_fastga(wd, "A", "B", threads=4))
-    ref = ol.oneview_records(os.path.join(wd, "ref.1aln"))
+    ref = ol.reference_run("oracle/scaffolded")
+    st = ref["counters"]
     gA = formats.genome_from_fasta(os.path.join(wd, "A.fasta"))
     gB = formats.genome_from_fasta(os.path.join(wd, "B.fasta"))
-    clen, names, scaf, sbeg = ol.read_gdb_ascii(os.path.join(wd, "B.1gdb"))
-    assert np.array_equal(clen, gB.clen) and np.array_equal(sbeg, gB.sbeg) and np.array_equal(scaf, gB.scaf)
+    gdb = ref["gdb_B"]
+    assert list(gB.clen) == gdb["clen"] and list(gB.sbeg) == gdb["sbeg"] and list(gB.scaf) == gdb["scaf"]
     r = ol.oracle_pipeline(gA, gB)
     assert (r["nseeds"], r["nhit"], r["nraw"], len(r["lines"])) == (st["seeds"], st["hits"], st["alns"], st["kept"])
-    assert r["lines"] == ref
+    assert len(r["lines"]) == ref["records"] and ol.md5_lines(r["lines"]) == ref["aln_md5"]
 
 
-@pytest.mark.skipif(not ol.have_ref(), reason="oracle/_ref not built")
 def test_written_1aln_is_read_by_reference_tools(tmp_path):
-    """SURVEY 8 a-16: a .1aln written by formats.write_1aln_ascii is accepted by the reference's
-    ONEview (same records back) and -- after ONEview -b adds the binary index the threaded readers
-    need -- by its ALNtoPAF next to the reference-made GDBs (same PAF as from the reference's own
-    .1aln)."""
+    """SURVEY 8 a-16: a .1aln written by formats.write_1aln_ascii carries the records of the
+    reference's own .1aln, in the text ONEview reads back (tests/golden/reference_runs.json).  Where
+    the reference tools are built, the file also goes through them: ONEview returns the same records
+    and -- after ONEview -b adds the binary index the threaded readers need -- ALNtoPAF, next to the
+    reference-made GDBs, gives the same PAF as from the reference's own .1aln."""
     A, B = synth.make_pair(41, 500_000, 3, 0.06, sv_every=40_000)
     wd = str(tmp_path)
     formats.write_fasta(os.path.join(wd, "A.fasta"), synth.scaffolds_of(A, "sa", 2))
     formats.write_fasta(os.path.join(wd, "B.fasta"), synth.scaffolds_of(B, "sb", 1))
-    ol.ref_fastga(wd, "A", "B", threads=4)
     gA = formats.genome_from_fasta(os.path.join(wd, "A.fasta"))
     gB = formats.genome_from_fasta(os.path.join(wd, "B.fasta"))
     r = ol.oracle_pipeline(gA, gB)
     formats.write_1aln_ascii(os.path.join(wd, "mine.1aln"), r["alns"], gA, gB, "./A.1gdb", "./B.1gdb", wd)
+    ref = ol.reference_run("oracle/written_1aln")
+    with open(os.path.join(wd, "mine.1aln")) as f:
+        mine = ol.records_from_text(f.read())
+    assert len(mine) == ref["records"] and ol.md5_lines(mine) == ref["aln_md5"]
+    if not ol.have_ref():
+        return
+    ol.ref_fastga(wd, "A", "B", threads=4)
     assert ol.oneview_records(os.path.join(wd, "mine.1aln")) == ol.oneview_records(os.path.join(wd, "ref.1aln"))
     paf_ref = sorted(ol.run_ref(["ALNtoPAF", "-T2", "ref"], cwd=wd).split("\n"))
     # the threaded converters need ONEcode's binary index: ONEview -b turns the ASCII file into it
@@ -192,39 +182,34 @@ def test_written_1aln_is_read_by_reference_tools(tmp_path):
     assert len(paf_ref) > 3 and paf_mine == paf_ref
 
 
+def _assert_reference_run(r, key):
+    ref = ol.reference_run(key)
+    assert r["nseeds"] == ref["counters"].get("seeds", 0)
+    assert len(r["lines"]) == ref["records"] and ol.md5_lines(r["lines"]) == ref["aln_md5"]
+
+
 import edge_cases  # noqa: E402
 
 
-@pytest.mark.skipif(not ol.have_ref(), reason="oracle/_ref not built")
 @pytest.mark.parametrize("name", sorted(edge_cases.CASES))
-def test_oracle_edge_cases_vs_live_reference(name, tmp_path):
-    """the oracle on the edge-case inputs of tests/edge_cases.py, against a live reference run"""
+def test_oracle_edge_cases_vs_live_reference(name):
+    """the oracle on the edge-case inputs of tests/edge_cases.py, against the reference's run on them"""
     A, B, threads, check = edge_cases.CASES[name]()
-    wd = str(tmp_path)
-    formats.write_fasta(os.path.join(wd, "A.fasta"), synth.scaffolds_of(A, "sa", 1))
-    formats.write_fasta(os.path.join(wd, "B.fasta"), synth.scaffolds_of(B, "sb", 1))
-    st = ol.parse_fastga_log(ol.ref_fastga(wd, "A", "B", threads=threads))
-    ref = ol.oneview_records(os.path.join(wd, "ref.1aln"))
     r = ol.oracle_pipeline(formats.genome_from_arrays(A), formats.genome_from_arrays(B))
-    assert r["nseeds"] == st.get("seeds", 0)
-    assert r["lines"] == ref
+    _assert_reference_run(r, "edge/" + name)
     check(r["alns"], r["nhit"])
 
 
-@pytest.mark.skipif(not ol.have_ref(), reason="oracle/_ref not built")
-def test_oracle_on_example_regions_vs_live_reference(tmp_path):
-    """the EXAMPLE regions fixture of the GPU regression test, oracle against a live reference run"""
-    z = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "example_regions.npz"))
-    A = [z["a%d" % i] for i in range(10)]
-    B = [z["b%d" % i] for i in range(10)]
-    wd = str(tmp_path)
-    formats.write_fasta(os.path.join(wd, "A.fasta"), synth.scaffolds_of(A, "sa", 1))
-    formats.write_fasta(os.path.join(wd, "B.fasta"), synth.scaffolds_of(B, "sb", 1))
-    st = ol.parse_fastga_log(ol.ref_fastga(wd, "A", "B", threads=4))
-    ref = ol.oneview_records(os.path.join(wd, "ref.1aln"))
+def example_regions():
+    z = np.load(os.path.join(ol.GOLDEN, "example_regions.npz"))
+    return [z["a%d" % i] for i in range(10)], [z["b%d" % i] for i in range(10)]
+
+
+def test_oracle_on_example_regions_vs_live_reference():
+    """the EXAMPLE regions fixture of the GPU regression test, oracle against the reference's run on it"""
+    A, B = example_regions()
     r = ol.oracle_pipeline(formats.genome_from_arrays(A), formats.genome_from_arrays(B))
-    assert r["nseeds"] == st.get("seeds", 0)
-    assert r["lines"] == ref
+    _assert_reference_run(r, "oracle/example_regions")
 
 
 def _self_genomes():
@@ -268,19 +253,16 @@ def _self_genomes():
     return out
 
 
-@pytest.mark.skipif(not ol.have_ref(), reason="oracle/_ref not built")
 @pytest.mark.parametrize("name", ["dup", "tandem61", "tandem62", "inverted_dup", "identical_contigs",
                                   "palindrome", "near_diagonal_repeats"])
-def test_oracle_self_mode_vs_live_reference(name, tmp_path):
+def test_oracle_self_mode_vs_live_reference(name):
     """SURVEY row a-7 groundwork: the oracle's SELF mode (self block rule, band borders for a contig
-    against itself) against `FastGA A` of the reference"""
+    against itself) against `FastGA A` of the reference (tests/golden/reference_runs.json)"""
     G = _self_genomes()[name]
-    wd = str(tmp_path)
-    formats.write_fasta(os.path.join(wd, "A.fasta"), synth.scaffolds_of(G, "sa", 1))
-    st = ol.parse_fastga_log(ol.ref_fastga(wd, "A", None, threads=4))
-    ref = ol.oneview_records(os.path.join(wd, "ref.1aln"))
+    ref = ol.reference_run("self/" + name)
+    st = ref["counters"]
     r = ol.oracle_pipeline_self(formats.genome_from_arrays(G))
     # every thread of the reference halves its own pair count (FastGA.c:1907): off by < #threads
     assert abs(r["nseeds"] // 2 - st["seeds"]) < 4
     assert r["nhit"] == st["hits"] and r["nraw"] == st["alns"]
-    assert r["lines"] == ref
+    assert len(r["lines"]) == ref["records"] and ol.md5_lines(r["lines"]) == ref["aln_md5"]
