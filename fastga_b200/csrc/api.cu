@@ -28,11 +28,11 @@ int fgb_syncmer_count_device(const void *d_seq, const long long *d_clen, const l
                              const int *d_crank, const int *d_tile_contig, const int *d_tile_start,
                              int ntiles, unsigned *d_tile_count, unsigned long long *d_buck1024,
                              unsigned long long *d_total, void *d_tmp, long long tmp_bytes,
-                             unsigned plo, unsigned phi, void *stream);
+                             int fwd_only, void *stream);
 int fgb_syncmer_emit_device(const void *d_seq, const long long *d_clen, const long long *d_woff,
                             const int *d_crank, const int *d_tile_contig, const int *d_tile_start,
-                            int ntiles, unsigned *d_tile_offset, void *d_records, unsigned plo,
-                            unsigned phi, void *stream);
+                            int ntiles, unsigned *d_tile_offset, void *d_records, int fwd_only,
+                            void *stream);
 int fgb_kix_index_device(const void *d_tab, long long n, unsigned *d_pstart, unsigned char *d_adj, void *stream);
 int fgb_ktab_export_device(const void *d_tab, long long n, int pbytes, int cbytes,
                            const long long *d_part_first, int nparts, void *d_out, void *stream);
@@ -43,7 +43,6 @@ int fgb_owner_count_device(const void *d_seeds, long long n, int p_ic, int ic_bi
                            int world, unsigned long long *d_cnt, void *stream);
 int fgb_owner_scatter_device(const void *d_seeds, long long n, int p_ic, int ic_bits, const int *d_owner, int nrc,
                              int world, unsigned long long *d_base, void *d_out, void *stream);
-int fgb_kmer_bins_device(const void *d_tab, long long n, int binshift, unsigned *d_bins, void *stream);
 int fgb_self_merge_device(const void *d_T, long long n, const unsigned *d_pstart, int freq,
                           int anti_bits, int band_bits, int jc_bits, int ic_bits,
                           long long amxpos, void *d_seeds, long long capacity,
@@ -57,25 +56,7 @@ int fgb_merge_device(const void *d_T1, long long n1, const void *d_T2, long long
                      unsigned long long *h_sumlen, void *stream);
 }
 
-static fgb_timings g_timings;
-
-struct stage_timer
-{ cudaEvent_t a, b; cudaStream_t st; float *dst;
-  stage_timer(float *d, cudaStream_t s) : st(s), dst(d)
-    { cudaEventCreate(&a); cudaEventCreate(&b); cudaEventRecord(a,st); }
-  ~stage_timer()
-    { cudaEventRecord(b,st); cudaEventSynchronize(b);
-      float ms = 0; cudaEventElapsedTime(&ms,a,b); *dst += ms;
-      cudaEventDestroy(a); cudaEventDestroy(b);
-    }
-};
-
-void fgb_timing_add(int which, float ms)
-{ if (which == 0) g_timings.triples_ms += ms;
-  else if (which == 1) { g_timings.extend_ms += ms; g_timings.extend_launches += 1; }
-  else if (which == 3) { g_timings.merge_ms += ms; g_timings.merge_launches += 1; }
-  else g_timings.d2h_ms += ms;
-}
+fgb_timings g_timings;
 
 void fgb_count_launch(int n) { g_timings.launches += n; }
 
@@ -148,6 +129,14 @@ extern "C" void fgb_timings_get(fgb_timings *out) { *out = g_timings; }
  *  Genome: the GDB as the path sees it (GDB.h:28-34 GDB_CONTIG {clen, boff} + the .bps image)
  **********************************************************************************************/
 
+extern "C" void fgb_genome_free(fgb_genome *g)
+{ cudaStream_t st = 0;
+  if (!g) return;
+  fgb_dfree(g->d_clen,st); fgb_dfree(g->d_woff,st); fgb_dfree(g->d_crank,st); fgb_dfree(g->d_perm,st);
+  fgb_dfree(g->d_seq,st); fgb_dfree(g->d_rseq,st);
+  delete g;
+}
+
 static const long long *g_sort_len;
 static int LSORT(const void *l, const void *r)          // GIXmake.c:1628-1633: decreasing length
 { int x = *((const int *) l), y = *((const int *) r);
@@ -159,7 +148,8 @@ extern "C" int fgb_genome_create(const unsigned char *bps, long long bps_bytes, 
                                  fgb_genome **out, void *stream)
 { cudaStream_t st = (cudaStream_t) stream;
   if (ncontig <= 0 || ncontig > 0x7fff) return FGB_ERR_LIMIT;   // contig rank is a 15-bit field
-  fgb_genome *g = new fgb_genome();
+  owner<fgb_genome> own(new fgb_genome(),fgb_genome_free);
+  fgb_genome *g = own.get();
   g->ncontig = ncontig;
   g->clen.assign(clen,clen+ncontig);
   g->boff.assign(boff,boff+ncontig);
@@ -167,7 +157,7 @@ extern "C" int fgb_genome_create(const unsigned char *bps, long long bps_bytes, 
   g->seqtot = 0; g->maxlen = 0;
   long long w = 2;                             // 16 zero bytes ahead of the first contig too
   for (int c = 0; c < ncontig; c++)
-    { if (clen[c] >= 0x7fffffffll) { delete g; return FGB_ERR_LIMIT; }
+    { if (clen[c] >= 0x7fffffffll) return FGB_ERR_LIMIT;
       g->woff[c] = w;
       w += ((clen[c] + 31) >> 5) + 2;          // zero pad so 64-bit window reads stay inside
       w = (w + 1) & ~1ll;                      // 16-byte alignment of every contig
@@ -185,6 +175,7 @@ extern "C" int fgb_genome_create(const unsigned char *bps, long long bps_bytes, 
 
   unsigned char *d_bps = NULL;
   long long *d_boff = NULL;
+  dev_scope S(st); S.own(d_bps); S.own(d_boff);
   CUDA_TRY(fgb_dmalloc((void **) &d_bps,bps_bytes + 16,st));
   CUDA_TRY(fgb_dmalloc((void **) &d_boff,sizeof(long long)*ncontig,st));
   CUDA_TRY(fgb_dmalloc((void **) &g->d_clen,sizeof(long long)*ncontig,st));
@@ -207,18 +198,9 @@ extern "C" int fgb_genome_create(const unsigned char *bps, long long bps_bytes, 
     rc = fgb_stage_genome_device(d_bps,d_boff,g->d_clen,g->d_woff,ncontig,w,g->d_seq,g->d_rseq,st);
   }
   CUDA_TRY(cudaStreamSynchronize(st));
-  fgb_dfree(d_bps,st); fgb_dfree(d_boff,st);
-  if (rc) { delete g; return rc; }
-  *out = g;
+  if (rc) return rc;
+  *out = own.release();
   return FGB_OK;
-}
-
-extern "C" void fgb_genome_free(fgb_genome *g)
-{ cudaStream_t st = 0;
-  if (!g) return;
-  fgb_dfree(g->d_clen,st); fgb_dfree(g->d_woff,st); fgb_dfree(g->d_crank,st); fgb_dfree(g->d_perm,st);
-  fgb_dfree(g->d_seq,st); fgb_dfree(g->d_rseq,st);
-  delete g;
 }
 
 extern "C" int fgb_genome_perm(const fgb_genome *g, int *perm_out)
@@ -257,44 +239,10 @@ static void gix_bytes(const fgb_genome *g, fgb_gix *x)        // GIXmake.c:1888-
 //  K1..K4: syncmer scan -> 128-bit records -> 10-pass byte radix sort on the 80-bit k-mer ->
 //  2^24 prefix index.
 
-#define GIX_FWD_ONLY 0x80000000u     // flag bit carried in `phi` down to syncmer_kernel
-#define GIX_NO_INDEX 0x40000000u     // table only: no prefix index, no LCP bytes (the T1 side of a merge reads neither)
-
-static int gix_build_range(const fgb_genome *g, unsigned plo, unsigned phi, fgb_gix **out, void *stream);
-
-//  a table handle (and, with it, its device blocks) is released on every way out of the call that
-//  builds it unless it was handed to the caller; likewise loose device blocks
-struct gix_scope
-{ fgb_gix *x;
-  explicit gix_scope(fgb_gix *p) : x(p) {}
-  fgb_gix *release() { fgb_gix *p = x; x = NULL; return p; }
-  ~gix_scope() { if (x != NULL) fgb_gix_free(x); }
-};
-struct blk_scope
-{ std::vector<void **> slots;
-  template<class T> void own(T *&p) { slots.push_back((void **) &p); }
-  ~blk_scope() { for (void **s : slots) if (*s != NULL) { fgb_dfree(*s,0); *s = NULL; } }
-};
-
-extern "C" int fgb_gix_build(const fgb_genome *g, fgb_gix **out, void *stream)
-{ return gix_build_range(g,0u,1u << 24,out,stream); }
-
-//  Forward-strand entries only: the table of the genome that supplies the adaptamers.  Reverse
-//  entries of T1 never seed (FastGA.c:921-928), so the fused path does not build, sort or read them.
-extern "C" int fgb_gix_build_forward(const fgb_genome *g, fgb_gix **out, void *stream)
-{ return gix_build_range(g,0u,(1u << 24) | GIX_FWD_ONLY,out,stream); }
-
-//  Only the k-mers whose 12-base prefix lies in [plo,phi): one rank's share of a table that is
-//  built cooperatively (every rank scans the genome, sorts 1/N of the records, the sorted shares
-//  concatenate in rank order -- fastga_b200/shard.py all-gathers them over NCCL).
-extern "C" int fgb_gix_build_range(const fgb_genome *g, unsigned plo, unsigned phi, fgb_gix **out, void *stream)
-{ if (plo > phi || phi > (1u << 24)) return FGB_ERR_ARG;
-  return gix_build_range(g,plo,phi,out,stream);
-}
-
 //  K1/K2: syncmer scan + record build of the contigs selected by `mask` (NULL: all) into a fresh
-//  device buffer of *n unsorted records (room for n+1).  *nrev = reverse entries left out (fwd-only).
-static int gix_scan(const fgb_genome *g, const unsigned char *mask, unsigned plo, unsigned phi_flags,
+//  device buffer of *n unsorted records (room for n+1).  fwd_only: forward-strand entries only,
+//  *nrev = reverse entries left out.
+static int gix_scan(const fgb_genome *g, const unsigned char *mask, bool fwd_only,
                     rec128 **d_recs, long long *n_out, long long *nrev, unsigned long long *buck1024, cudaStream_t st)
 { int T = fgb_sc_tile();
   std::vector<int> tc, ts;
@@ -306,86 +254,93 @@ static int gix_scan(const fgb_genome *g, const unsigned char *mask, unsigned plo
   int *d_tc = NULL, *d_ts = NULL; unsigned *d_cnt = NULL;
   u64 *d_buck = NULL, *d_total = NULL; void *d_tmp = NULL;
   rec128 *d_a = NULL;
+  dev_scope S(st); S.own(d_tc); S.own(d_ts); S.own(d_cnt); S.own(d_buck); S.own(d_total); S.own(d_tmp); S.own(d_a);
   long long tmpb = fgb_dev_scan_tmp_bytes(ntiles);
-  int rc = FGB_OK;
+  int rc;
   u64 total = 0, rdropped = 0;
-#define GS_TRY(call) do { if ((call) != cudaSuccess) { rc = FGB_ERR_CUDA; goto done; } } while (0)
-  GS_TRY(fgb_dmalloc((void **) &d_tc,sizeof(int)*(ntiles+1),st));
-  GS_TRY(fgb_dmalloc((void **) &d_ts,sizeof(int)*(ntiles+1),st));
-  GS_TRY(fgb_dmalloc((void **) &d_cnt,sizeof(unsigned)*(ntiles+1),st));
-  GS_TRY(fgb_dmalloc((void **) &d_buck,8*1025,st));
-  GS_TRY(fgb_dmalloc((void **) &d_total,8,st));
-  GS_TRY(fgb_dmalloc((void **) &d_tmp,tmpb,st));
-  GS_TRY(cudaMemcpyAsync(d_tc,tc.data(),sizeof(int)*ntiles,cudaMemcpyHostToDevice,st));
-  GS_TRY(cudaMemcpyAsync(d_ts,ts.data(),sizeof(int)*ntiles,cudaMemcpyHostToDevice,st));
+  CUDA_TRY(fgb_dmalloc((void **) &d_tc,sizeof(int)*(ntiles+1),st));
+  CUDA_TRY(fgb_dmalloc((void **) &d_ts,sizeof(int)*(ntiles+1),st));
+  CUDA_TRY(fgb_dmalloc((void **) &d_cnt,sizeof(unsigned)*(ntiles+1),st));
+  CUDA_TRY(fgb_dmalloc((void **) &d_buck,8*1025,st));
+  CUDA_TRY(fgb_dmalloc((void **) &d_total,8,st));
+  CUDA_TRY(fgb_dmalloc((void **) &d_tmp,tmpb,st));
+  CUDA_TRY(cudaMemcpyAsync(d_tc,tc.data(),sizeof(int)*ntiles,cudaMemcpyHostToDevice,st));
+  CUDA_TRY(cudaMemcpyAsync(d_ts,ts.data(),sizeof(int)*ntiles,cudaMemcpyHostToDevice,st));
   { stage_timer t(&g_timings.scan_ms,st);
     rc = fgb_syncmer_count_device(g->d_seq,g->d_clen,g->d_woff,g->d_crank,d_tc,d_ts,ntiles,d_cnt,
-                                  d_buck,d_total,d_tmp,tmpb,plo,phi_flags,st);
-    if (rc) goto done;
-    GS_TRY(cudaMemcpyAsync(&total,d_total,8,cudaMemcpyDeviceToHost,st));
-    if (buck1024) GS_TRY(cudaMemcpyAsync(buck1024,d_buck,8*1024,cudaMemcpyDeviceToHost,st));
-    GS_TRY(cudaMemcpyAsync(&rdropped,d_buck + 1024,8,cudaMemcpyDeviceToHost,st));
-    GS_TRY(cudaStreamSynchronize(st));
+                                  d_buck,d_total,d_tmp,tmpb,fwd_only,st);
+    if (rc) return rc;
+    CUDA_TRY(cudaMemcpyAsync(&total,d_total,8,cudaMemcpyDeviceToHost,st));
+    if (buck1024) CUDA_TRY(cudaMemcpyAsync(buck1024,d_buck,8*1024,cudaMemcpyDeviceToHost,st));
+    CUDA_TRY(cudaMemcpyAsync(&rdropped,d_buck + 1024,8,cudaMemcpyDeviceToHost,st));
+    CUDA_TRY(cudaStreamSynchronize(st));
   }
-  if (total >= 0xfffffff0ull) { rc = FGB_ERR_LIMIT; goto done; }
-  GS_TRY(fgb_dmalloc((void **) &d_a,sizeof(rec128)*(total+1),st));
+  if (total >= 0xfffffff0ull) return FGB_ERR_LIMIT;
+  CUDA_TRY(fgb_dmalloc((void **) &d_a,sizeof(rec128)*(total+1),st));
   { stage_timer t(&g_timings.scan_ms,st);
-    rc = fgb_syncmer_emit_device(g->d_seq,g->d_clen,g->d_woff,g->d_crank,d_tc,d_ts,ntiles,d_cnt,d_a,plo,phi_flags,st);
+    rc = fgb_syncmer_emit_device(g->d_seq,g->d_clen,g->d_woff,g->d_crank,d_tc,d_ts,ntiles,d_cnt,d_a,fwd_only,st);
   }
-  if (rc == FGB_OK && cudaStreamSynchronize(st) != cudaSuccess) rc = FGB_ERR_CUDA;   // tc/ts must outlive the copies
-done:
-#undef GS_TRY
-  fgb_dfree(d_tc,st); fgb_dfree(d_ts,st); fgb_dfree(d_cnt,st); fgb_dfree(d_buck,st); fgb_dfree(d_total,st); fgb_dfree(d_tmp,st);
-  if (rc) { fgb_dfree(d_a,st); return rc; }
-  *d_recs = d_a; *n_out = (long long) total; *nrev = (long long) rdropped;
+  if (rc) return rc;
+  CUDA_TRY(cudaStreamSynchronize(st));                      // tc/ts must outlive the copies
+  *d_recs = d_a; d_a = NULL;                                // handed to the caller
+  *n_out = (long long) total; *nrev = (long long) rdropped;
   return FGB_OK;
 }
 
-//  K3/K4: sorts the records in d_a (consumed: it ends up inside the handle or is released) whose
-//  12-base prefixes lie in [plo,phi), builds the prefix index and the LCP bytes.
-static int gix_finish(fgb_gix *x, rec128 *d_a, long long n, unsigned plo, unsigned phi, cudaStream_t st, bool index = true)
+//  K3/K4: sorts the records in d_a whose 12-base prefixes lie in [plo,phi) and, with `index`, builds
+//  the prefix index and the LCP bytes.  d_a is consumed: it ends up inside the handle or is released,
+//  and the caller's pointer is cleared either way.
+static int gix_finish(fgb_gix *x, rec128 *&d_a, long long n, unsigned plo, unsigned phi, bool index, cudaStream_t st)
 { rec128 *d_b = NULL; void *d_stmp = NULL;
+  dev_scope S(st); S.own(d_a); S.own(d_b); S.own(d_stmp);
   long long stmpb = fgb_sort128_tmp_bytes(n);
-  int rc = FGB_OK, inb = 0;
+  int rc, inb = 0;
   x->n = n;
-  if (fgb_dmalloc((void **) &d_b,sizeof(rec128)*(n+1),st) != cudaSuccess ||
-      fgb_dmalloc((void **) &d_stmp,stmpb,st) != cudaSuccess ||
-      (index && fgb_dmalloc((void **) &x->d_pstart,sizeof(unsigned)*((1<<24)+1+8),st) != cudaSuccess) ||
-      (index && fgb_dmalloc((void **) &x->d_adj,(size_t) n + 32,st) != cudaSuccess))
-    rc = FGB_ERR_CUDA;
-  if (!rc)
-    { stage_timer t(&g_timings.ksort_ms,st);
-      rc = fgb_kmer_sort_range_device(d_a,d_b,n,plo,phi,d_stmp,stmpb,&inb,st);
+  CUDA_TRY(fgb_dmalloc((void **) &d_b,sizeof(rec128)*(n+1),st));
+  CUDA_TRY(fgb_dmalloc((void **) &d_stmp,stmpb,st));
+  if (index)
+    { CUDA_TRY(fgb_dmalloc((void **) &x->d_pstart,sizeof(unsigned)*((1<<24)+1+8),st));
+      CUDA_TRY(fgb_dmalloc((void **) &x->d_adj,(size_t) n + 32,st));
     }
-  if (!rc)
-    { x->d_tab = inb ? d_b : d_a;
-      if (inb) d_b = NULL; else d_a = NULL;
-      if (index)
-        { stage_timer t(&g_timings.index_ms,st);
-          rc = fgb_kix_index_device(x->d_tab,n,x->d_pstart,x->d_adj,st);
-        }
+  { stage_timer t(&g_timings.ksort_ms,st);
+    rc = fgb_kmer_sort_range_device(d_a,d_b,n,plo,phi,d_stmp,stmpb,&inb,st);
+  }
+  if (rc) return rc;
+  x->d_tab = inb ? d_b : d_a;
+  if (inb) d_b = NULL; else d_a = NULL;                     // ownership moved to the handle
+  if (index)
+    { stage_timer t(&g_timings.index_ms,st);
+      rc = fgb_kix_index_device(x->d_tab,n,x->d_pstart,x->d_adj,st);
     }
-  if (!rc && cudaStreamSynchronize(st) != cudaSuccess) rc = FGB_ERR_CUDA;
-  fgb_dfree(d_a,st); fgb_dfree(d_b,st); fgb_dfree(d_stmp,st);
-  return rc;
+  if (rc) return rc;
+  CUDA_TRY(cudaStreamSynchronize(st));
+  return FGB_OK;
 }
 
-static int gix_build_range(const fgb_genome *g, unsigned plo, unsigned phi_flags, fgb_gix **out, void *stream)
-{ cudaStream_t st = (cudaStream_t) stream;
-  const bool index = !(phi_flags & GIX_NO_INDEX);
-  phi_flags &= ~GIX_NO_INDEX;
-  const unsigned phi = phi_flags & ~GIX_FWD_ONLY;
-  fgb_gix *x = new fgb_gix();
+//  fwd_only: forward-strand entries only; index: false = the table alone, no prefix index and no LCP
+//  bytes (the T1 side of a merge reads neither)
+static int gix_build(const fgb_genome *g, bool fwd_only, bool index, fgb_gix **out, cudaStream_t st)
+{ owner<fgb_gix> own(new fgb_gix(),fgb_gix_free);
+  fgb_gix *x = own.get();
   gix_bytes(g,x);
   x->ncontig = g->ncontig;
-  x->fwd_only = (phi_flags & GIX_FWD_ONLY) ? 1 : 0;
+  x->fwd_only = fwd_only ? 1 : 0;
   rec128 *d_a = NULL; long long n = 0, nrev = 0;
-  int rc = gix_scan(g,NULL,plo,phi_flags,&d_a,&n,&nrev,x->buck1024,st);
-  if (!rc) { x->n_both = n + nrev; rc = gix_finish(x,d_a,n,plo,phi,st,index); }
-  if (rc) { fgb_gix_free(x); return rc; }
-  *out = x;
+  int rc = gix_scan(g,NULL,fwd_only,&d_a,&n,&nrev,x->buck1024,st);
+  if (rc) return rc;
+  x->n_both = n + nrev;
+  if ((rc = gix_finish(x,d_a,n,0u,1u << 24,index,st))) return rc;
+  *out = own.release();
   return FGB_OK;
 }
+
+extern "C" int fgb_gix_build(const fgb_genome *g, fgb_gix **out, void *stream)
+{ return gix_build(g,false,true,out,(cudaStream_t) stream); }
+
+//  Forward-strand entries only: the table of the genome that supplies the adaptamers.  Reverse
+//  entries of T1 never seed (FastGA.c:921-928), so the fused path does not build, sort or read them.
+extern "C" int fgb_gix_build_forward(const fgb_genome *g, fgb_gix **out, void *stream)
+{ return gix_build(g,true,true,out,(cudaStream_t) stream); }
 
 /***********************************************************************************************
  *  Building blocks of the k-mer-space sharded path (several GPUs, fastga_b200/shard.py): every rank
@@ -403,34 +358,9 @@ extern "C" void fgb_device_free(void *p) { fgb_dfree(p,0); }
 extern "C" int fgb_kmers_scan(const fgb_genome *g, const unsigned char *mask, int fwd_only,
                               void **d_recs, long long *n, void *stream)
 { rec128 *d = NULL; long long nrev = 0;
-  int rc = gix_scan(g,mask,0u,(1u << 24) | (fwd_only ? GIX_FWD_ONLY : 0u),&d,n,&nrev,NULL,(cudaStream_t) stream);
+  int rc = gix_scan(g,mask,fwd_only != 0,&d,n,&nrev,NULL,(cudaStream_t) stream);
   if (rc) return rc;
   *d_recs = d;
-  return FGB_OK;
-}
-
-//  records grouped by the top byte of the k-mer (its first four bases): d_out[bounds[b] .. bounds[b+1])
-//  holds those with top byte b, b = 0..255.  One Onesweep pass; the owner of a record is any
-//  monotone function of that byte, so the send blocks of an all-to-all are contiguous.
-extern "C" int fgb_records_group_by_top_byte(void *d_recs, long long n, void *d_out, long long *bounds257,
-                                             void *stream)
-{ cudaStream_t st = (cudaStream_t) stream;
-  for (int b = 0; b <= 256; b++) bounds257[b] = 0;
-  if (n <= 0) return FGB_OK;
-  void *d_tmp = NULL; unsigned *d_bins = NULL;
-  long long tmpb = fgb_sort128_tmp_bytes(n);
-  int rc = FGB_OK, inb = 0;
-  std::vector<unsigned> bins(65537);
-  if (fgb_dmalloc(&d_tmp,tmpb,st) != cudaSuccess || fgb_dmalloc((void **) &d_bins,sizeof(unsigned)*65537,st) != cudaSuccess)
-    rc = FGB_ERR_CUDA;
-  if (!rc) rc = fgb_sort128_device(d_recs,d_out,n,15,16,d_tmp,tmpb,&inb,st);
-  if (!rc && !inb && cudaMemcpyAsync(d_out,d_recs,sizeof(rec128)*n,cudaMemcpyDeviceToDevice,st) != cudaSuccess) rc = FGB_ERR_CUDA;
-  if (!rc) rc = fgb_kmer_bins_device(d_out,n,56,d_bins,st);
-  if (!rc && (cudaMemcpyAsync(bins.data(),d_bins,sizeof(unsigned)*65537,cudaMemcpyDeviceToHost,st) != cudaSuccess ||
-              cudaStreamSynchronize(st) != cudaSuccess)) rc = FGB_ERR_CUDA;
-  fgb_dfree(d_tmp,st); fgb_dfree(d_bins,st);
-  if (rc) return rc;
-  for (int b = 0; b <= 256; b++) bounds257[b] = bins[b];
   return FGB_OK;
 }
 
@@ -440,49 +370,21 @@ extern "C" int fgb_gix_from_records(const void *d_recs, long long n, unsigned pl
                                     int post_bytes, int cont_bytes, int ncontig, fgb_gix **out, void *stream)
 { cudaStream_t st = (cudaStream_t) stream;
   if (n < 0 || n >= 0xfffffff0ll || plo >= phi || phi > (1u << 24)) return FGB_ERR_ARG;
-  fgb_gix *x = new fgb_gix();
+  owner<fgb_gix> own(new fgb_gix(),fgb_gix_free);
+  fgb_gix *x = own.get();
   x->n_both = n; x->post_bytes = post_bytes; x->cont_bytes = cont_bytes; x->ncontig = ncontig;
   x->fwd_only = fwd_only ? 1 : 0;
   rec128 *d_a = NULL;
-  int rc = FGB_OK;
-  if (fgb_dmalloc((void **) &d_a,sizeof(rec128)*(n+1),st) != cudaSuccess) rc = FGB_ERR_CUDA;
-  if (!rc && n > 0 && cudaMemcpyAsync(d_a,d_recs,sizeof(rec128)*n,cudaMemcpyDeviceToDevice,st) != cudaSuccess) rc = FGB_ERR_CUDA;
-  if (!rc) rc = gix_finish(x,d_a,n,plo,phi,st); else fgb_dfree(d_a,st);
-  if (rc) { fgb_gix_free(x); return rc; }
-  *out = x;
-  return FGB_OK;
-}
-
-extern "C" long long fgb_gix_size(const fgb_gix *x) { return x->n; }
-
-//  device-to-device copy of the sorted records into a caller-owned device buffer (n x 16 bytes)
-extern "C" int fgb_gix_copy_table(const fgb_gix *x, void *d_dst, void *stream)
-{ CUDA_TRY(cudaMemcpyAsync(d_dst,x->d_tab,sizeof(rec128)*x->n,cudaMemcpyDeviceToDevice,(cudaStream_t) stream));
-  CUDA_TRY(cudaStreamSynchronize((cudaStream_t) stream));
-  return FGB_OK;
-}
-
-//  A GIX over sorted device-layout records that already sit in device memory (copied).
-extern "C" int fgb_gix_from_device(const void *d_tab, long long n, int post_bytes, int cont_bytes,
-                                   int ncontig, fgb_gix **out, void *stream)
-{ cudaStream_t st = (cudaStream_t) stream;
-  if (n >= 0xfffffff0ll) return FGB_ERR_LIMIT;
-  fgb_gix *x = new fgb_gix();
-  gix_scope own(x);
-  x->n = n; x->n_both = n; x->post_bytes = post_bytes; x->cont_bytes = cont_bytes; x->ncontig = ncontig;
-  CUDA_TRY(fgb_dmalloc((void **) &x->d_tab,sizeof(rec128)*(n+1),st));
-  CUDA_TRY(fgb_dmalloc((void **) &x->d_pstart,sizeof(unsigned)*((1<<24)+1+8),st));
-  CUDA_TRY(fgb_dmalloc((void **) &x->d_adj,(size_t) x->n + 32,st));
-  CUDA_TRY(cudaMemcpyAsync(x->d_tab,d_tab,sizeof(rec128)*n,cudaMemcpyDeviceToDevice,st));
-  int rc;
-  { stage_timer t(&g_timings.index_ms,st);
-    rc = fgb_kix_index_device(x->d_tab,n,x->d_pstart,x->d_adj,st);
-  }
-  CUDA_TRY(cudaStreamSynchronize(st));
+  dev_scope S(st); S.own(d_a);
+  CUDA_TRY(fgb_dmalloc((void **) &d_a,sizeof(rec128)*(n+1),st));
+  if (n > 0) CUDA_TRY(cudaMemcpyAsync(d_a,d_recs,sizeof(rec128)*n,cudaMemcpyDeviceToDevice,st));
+  int rc = gix_finish(x,d_a,n,plo,phi,true,st);
   if (rc) return rc;
   *out = own.release();
   return FGB_OK;
 }
+
+extern "C" long long fgb_gix_size(const fgb_gix *x) { return x->n; }
 extern "C" int fgb_gix_post_bytes(const fgb_gix *x) { return x->post_bytes; }
 extern "C" int fgb_gix_cont_bytes(const fgb_gix *x) { return x->cont_bytes; }
 
@@ -494,25 +396,6 @@ extern "C" int fgb_gix_download(const fgb_gix *x, void *tab /* n x 16 B */, unsi
   return FGB_OK;
 }
 
-//  A GIX from host-side device-layout records (sorted) -- used to feed tables from elsewhere.
-extern "C" int fgb_gix_upload(const void *tab, long long n, int post_bytes, int cont_bytes,
-                              int ncontig, fgb_gix **out, void *stream)
-{ cudaStream_t st = (cudaStream_t) stream;
-  if (n >= 0xfffffff0ll) return FGB_ERR_LIMIT;
-  fgb_gix *x = new fgb_gix();
-  gix_scope own(x);
-  x->n = n; x->n_both = n; x->post_bytes = post_bytes; x->cont_bytes = cont_bytes; x->ncontig = ncontig;
-  CUDA_TRY(fgb_dmalloc((void **) &x->d_tab,sizeof(rec128)*(n+1),st));
-  CUDA_TRY(fgb_dmalloc((void **) &x->d_pstart,sizeof(unsigned)*((1<<24)+1+8),st));
-  CUDA_TRY(fgb_dmalloc((void **) &x->d_adj,(size_t) x->n + 32,st));
-  CUDA_TRY(cudaMemcpyAsync(x->d_tab,tab,sizeof(rec128)*n,cudaMemcpyHostToDevice,st));
-  int rc = fgb_kix_index_device(x->d_tab,n,x->d_pstart,x->d_adj,st);
-  CUDA_TRY(cudaStreamSynchronize(st));
-  if (rc) return rc;
-  *out = own.release();
-  return FGB_OK;
-}
-
 //  A GIX from the reference's on-disk form: concatenated .ktab entries (all parts, in order) and
 //  the stub's cumulative 2^24 index (libfastk.c:815-840).
 extern "C" int fgb_gix_import_ktab(const unsigned char *entries, long long n, int post_bytes,
@@ -520,12 +403,12 @@ extern "C" int fgb_gix_import_ktab(const unsigned char *entries, long long n, in
                                    fgb_gix **out, void *stream)
 { cudaStream_t st = (cudaStream_t) stream;
   if (n >= 0xfffffff0ll || post_bytes > 4 || cont_bytes > 2) return FGB_ERR_LIMIT;
-  fgb_gix *x = new fgb_gix();
-  gix_scope own(x);
+  owner<fgb_gix> own(new fgb_gix(),fgb_gix_free);
+  fgb_gix *x = own.get();
   x->n = n; x->n_both = n; x->post_bytes = post_bytes; x->cont_bytes = cont_bytes; x->ncontig = ncontig;
   long long E = 9 + post_bytes + cont_bytes;
   unsigned char *d_ent = NULL; long long *d_index = NULL;
-  blk_scope B; B.own(d_ent); B.own(d_index);
+  dev_scope S(st); S.own(d_ent); S.own(d_index);
   CUDA_TRY(fgb_dmalloc((void **) &d_ent,E*n + 16,st));
   CUDA_TRY(fgb_dmalloc((void **) &d_index,8ll<<24,st));
   CUDA_TRY(fgb_dmalloc((void **) &x->d_tab,sizeof(rec128)*(n+1),st));
@@ -548,7 +431,7 @@ extern "C" int fgb_gix_export_ktab(const fgb_gix *x, const long long *part_first
 { cudaStream_t st = (cudaStream_t) stream;
   long long E = 9 + x->post_bytes + x->cont_bytes;
   unsigned char *d_out = NULL; long long *d_pf = NULL;
-  blk_scope B; B.own(d_out); B.own(d_pf);
+  dev_scope S(st); S.own(d_out); S.own(d_pf);
   CUDA_TRY(fgb_dmalloc((void **) &d_out,E*x->n + 16,st));
   CUDA_TRY(fgb_dmalloc((void **) &d_pf,8*(nparts+1),st));
   CUDA_TRY(cudaMemcpyAsync(d_pf,part_first,8*nparts,cudaMemcpyHostToDevice,st));
@@ -598,72 +481,66 @@ static int seeds_merge_impl(const fgb_gix *x1, const fgb_gix *x2, long long amxp
                             bool self, const seed_bits &L, rec128 **d_out, long long *nseeds_out,
                             long long *sumlen_out, long long *n1m_out, cudaStream_t st)
 { if (self && x1->fwd_only) return FGB_ERR_ARG;                // SELF mode needs both strands
-  //  every device block of this call is released on every exit path
   u64 *d_counters = NULL; rec128 *d_fwd = NULL, *d_a = NULL;
-  int rc = FGB_OK;
+  dev_scope S(st); S.own(d_counters); S.own(d_fwd); S.own(d_a);
+  int rc;
   u64 nseeds = 0, sumlen = 0;
   //  the adaptamer side must be a forward-strand table (reverse entries never seed): a both-strand
   //  table (imported .ktab, fgb_gix_build) is compacted once; the fused path builds it forward-only
   const rec128 *t1 = x1->d_tab; long long n1 = x1->n;
-#define SF_TRY(call) do { if ((call) != cudaSuccess) { rc = FGB_ERR_CUDA; goto done; } } while (0)
-  SF_TRY(fgb_dmalloc((void **) &d_counters,16,st));
+  CUDA_TRY(fgb_dmalloc((void **) &d_counters,16,st));
   if (!self && !x1->fwd_only && n1 > 0)
-    { SF_TRY(fgb_dmalloc((void **) &d_fwd,sizeof(rec128)*(n1+1),st));
-      if ((rc = fgb_forward_view_device(x1->d_tab,n1,d_fwd,&n1,st))) goto done;
+    { CUDA_TRY(fgb_dmalloc((void **) &d_fwd,sizeof(rec128)*(n1+1),st));
+      if ((rc = fgb_forward_view_device(x1->d_tab,n1,d_fwd,&n1,st))) return rc;
       t1 = d_fwd;
     }
-  { long long cap = (self ? 2*x1->n : 2*n1 + (n1 >> 1)) + 1024;
-    for (int attempt = 0; ; attempt++)
-      { SF_TRY(fgb_dmalloc((void **) &d_a,sizeof(rec128)*(cap+1),st));
-        if (self)
-          rc = fgb_self_merge_device(x1->d_tab,x1->n,x1->d_pstart,freq,L.anti,L.band,L.jc,L.ic,amxpos,
-                                     d_a,cap,d_counters,&nseeds,&sumlen,st);
-        else
-          rc = fgb_merge_device(t1,n1,x2->d_tab,x2->n,x2->d_pstart,x2->d_adj,freq,L.anti,L.band,L.jc,L.ic,
-                                amxpos,bmxpos,d_a,cap,d_counters,&nseeds,&sumlen,st);
-        if (rc == FGB_OK) break;
-        fgb_dfree(d_a,st); d_a = NULL;
-        if (rc != FGB_ERR_OVERFLOW || attempt > 0) goto done;
-        cap = (long long) nseeds + 1024;
-        g_timings.merge_ms = 0; g_timings.merge_launches = 0;   // only the successful launch is reported
-      }
-  }
-  if (nseeds >= 0xfffffff0ull) rc = FGB_ERR_LIMIT;
-done:
-#undef SF_TRY
-  fgb_dfree(d_counters,st); fgb_dfree(d_fwd,st);
-  if (rc) { fgb_dfree(d_a,st); return rc; }
-  *d_out = d_a; *nseeds_out = (long long) nseeds; *sumlen_out = (long long) sumlen; *n1m_out = n1;
+  long long cap = (self ? 2*x1->n : 2*n1 + (n1 >> 1)) + 1024;
+  for (int attempt = 0; ; attempt++)
+    { CUDA_TRY(fgb_dmalloc((void **) &d_a,sizeof(rec128)*(cap+1),st));
+      if (self)
+        rc = fgb_self_merge_device(x1->d_tab,x1->n,x1->d_pstart,freq,L.anti,L.band,L.jc,L.ic,amxpos,
+                                   d_a,cap,d_counters,&nseeds,&sumlen,st);
+      else
+        rc = fgb_merge_device(t1,n1,x2->d_tab,x2->n,x2->d_pstart,x2->d_adj,freq,L.anti,L.band,L.jc,L.ic,
+                              amxpos,bmxpos,d_a,cap,d_counters,&nseeds,&sumlen,st);
+      if (rc == FGB_OK) break;
+      fgb_dfree(d_a,st); d_a = NULL;                          // the retry allocates it anew
+      if (rc != FGB_ERR_OVERFLOW || attempt > 0) return rc;
+      cap = (long long) nseeds + 1024;
+      g_timings.merge_ms = 0; g_timings.merge_launches = 0;   // only the successful launch is reported
+    }
+  if (nseeds >= 0xfffffff0ull) return FGB_ERR_LIMIT;
+  *d_out = d_a; d_a = NULL;                                   // handed to the caller
+  *nseeds_out = (long long) nseeds; *sumlen_out = (long long) sumlen; *n1m_out = n1;
   return FGB_OK;
 }
 
-//  K6: sorts n seed records in d_a (consumed) into a handle
-static int seeds_sort_impl(rec128 *d_a, long long n, const seed_bits &L, long long amxpos, long long bmxpos,
+//  K6: sorts n seed records in d_a into a handle.  d_a is consumed: it ends up inside the handle or
+//  is released, and the caller's pointer is cleared either way.
+static int seeds_sort_impl(rec128 *&d_a, long long n, const seed_bits &L, long long amxpos, long long bmxpos,
                            bool self, long long sumlen, long long n1m, fgb_seeds **out, cudaStream_t st)
-{ rec128 *d_b = NULL; void *d_tmp = NULL;
-  fgb_seeds *s = new fgb_seeds();
+{ owner<fgb_seeds> own(new fgb_seeds(),fgb_seeds_free);
+  rec128 *d_b = NULL; void *d_tmp = NULL;
+  dev_scope S(st); S.own(d_a); S.own(d_b); S.own(d_tmp);
+  fgb_seeds *s = own.get();
   s->self_mode = self ? 1 : 0;
   s->anti_bits = L.anti; s->band_bits = L.band; s->jc_bits = L.jc; s->ic_bits = L.ic;
   s->amxpos = amxpos; s->bmxpos = bmxpos;
   s->n = n; s->sumlen = sumlen; s->n1_merged = n1m;
   long long tmpb = fgb_sort128_tmp_bytes(n);
-  int rc = FGB_OK, inb = 0;
-  if (fgb_dmalloc((void **) &d_b,sizeof(rec128)*(n+1),st) != cudaSuccess ||
-      fgb_dmalloc((void **) &d_tmp,tmpb,st) != cudaSuccess) rc = FGB_ERR_CUDA;
-  if (!rc)
-    { stage_timer t(&g_timings.ssort_ms,st);
-      //  from bit 6: the lcp field (bits 0..5) cannot break a tie -- two seeds that agree on strand,
-      //  contigs, band, anti-diagonal and diagonal remainder are the same pair of positions
-      rc = fgb_sort128_bits_device(d_a,d_b,n,6,L.key,d_tmp,tmpb,&inb,st);
-    }
-  if (!rc && cudaStreamSynchronize(st) != cudaSuccess) rc = FGB_ERR_CUDA;
-  if (!rc)
-    { s->d_rec = inb ? d_b : d_a;
-      if (inb) d_b = NULL; else d_a = NULL;                     // ownership moved to the handle
-    }
-  fgb_dfree(d_a,st); fgb_dfree(d_b,st); fgb_dfree(d_tmp,st);
-  if (rc) { delete s; return rc; }
-  *out = s;
+  int rc, inb = 0;
+  CUDA_TRY(fgb_dmalloc((void **) &d_b,sizeof(rec128)*(n+1),st));
+  CUDA_TRY(fgb_dmalloc((void **) &d_tmp,tmpb,st));
+  { stage_timer t(&g_timings.ssort_ms,st);
+    //  from bit 6: the lcp field (bits 0..5) cannot break a tie -- two seeds that agree on strand,
+    //  contigs, band, anti-diagonal and diagonal remainder are the same pair of positions
+    rc = fgb_sort128_bits_device(d_a,d_b,n,6,L.key,d_tmp,tmpb,&inb,st);
+  }
+  if (rc) return rc;
+  CUDA_TRY(cudaStreamSynchronize(st));
+  s->d_rec = inb ? d_b : d_a;
+  if (inb) d_b = NULL; else d_a = NULL;                       // ownership moved to the handle
+  *out = own.release();
   return FGB_OK;
 }
 
@@ -695,70 +572,44 @@ extern "C" int fgb_seeds_merge(const fgb_gix *x1, const fgb_gix *x2, long long a
   return FGB_OK;
 }
 
-//  seeds grouped by the rank that owns their A-contig: owner[r] for contig RANK r (the icont field);
-//  d_out[bounds[w] .. bounds[w+1]) are the seeds of owner w.  Count + scatter, order inside a group free.
-extern "C" int fgb_seeds_group_by_owner(const void *d_seeds, long long n, const int *bits, const int *owner,
-                                        int nrank_contigs, int world, void *d_out, long long *bounds,
-                                        void *stream)
-{ cudaStream_t st = (cudaStream_t) stream;
-  if (world < 1 || world > 64) return FGB_ERR_ARG;
+//  d_out[bounds[w] .. bounds[w+1]) are the records with owner[f] == w, f = the field_bits wide field
+//  at bit field_pos of the record (f >= nowner: owner 0).  Count + scatter, order inside a group free.
+static int group_by_owner(const void *d_in, long long n, int field_pos, int field_bits, const int *owner,
+                          int nowner, int world, void *d_out, long long *bounds, cudaStream_t st)
+{ if (world < 1 || world > 64) return FGB_ERR_ARG;
   for (int w = 0; w <= world; w++) bounds[w] = 0;
   if (n <= 0) return FGB_OK;
   int *d_owner = NULL; u64 *d_cnt = NULL;
-  int rc = FGB_OK;
+  dev_scope S(st); S.own(d_owner); S.own(d_cnt);
+  int rc;
   u64 cnt[64], base[65];
-  const int p_ic = 12 + bits[0] + bits[1] + bits[2];
-  if (fgb_dmalloc((void **) &d_owner,sizeof(int)*(size_t) nrank_contigs,st) != cudaSuccess ||
-      fgb_dmalloc((void **) &d_cnt,8*64*2,st) != cudaSuccess) rc = FGB_ERR_CUDA;
-  if (!rc && (cudaMemcpyAsync(d_owner,owner,sizeof(int)*(size_t) nrank_contigs,cudaMemcpyHostToDevice,st) != cudaSuccess ||
-              cudaMemsetAsync(d_cnt,0,8*64*2,st) != cudaSuccess)) rc = FGB_ERR_CUDA;
-  if (!rc) rc = fgb_owner_count_device(d_seeds,n,p_ic,bits[3],d_owner,nrank_contigs,world,d_cnt,st);
-  if (!rc && (cudaMemcpyAsync(cnt,d_cnt,8*64,cudaMemcpyDeviceToHost,st) != cudaSuccess ||
-              cudaStreamSynchronize(st) != cudaSuccess)) rc = FGB_ERR_CUDA;
-  if (!rc)
-    { base[0] = 0;
-      for (int w = 0; w < world; w++) base[w+1] = base[w] + cnt[w];
-      if (cudaMemcpyAsync(d_cnt + 64,base,8*64,cudaMemcpyHostToDevice,st) != cudaSuccess) rc = FGB_ERR_CUDA;
-    }
-  if (!rc) rc = fgb_owner_scatter_device(d_seeds,n,p_ic,bits[3],d_owner,nrank_contigs,world,d_cnt + 64,d_out,st);
-  if (!rc && cudaStreamSynchronize(st) != cudaSuccess) rc = FGB_ERR_CUDA;
-  fgb_dfree(d_owner,st); fgb_dfree(d_cnt,st);
-  if (rc) return rc;
+  CUDA_TRY(fgb_dmalloc((void **) &d_owner,sizeof(int)*(size_t) nowner,st));
+  CUDA_TRY(fgb_dmalloc((void **) &d_cnt,8*64*2,st));
+  CUDA_TRY(cudaMemcpyAsync(d_owner,owner,sizeof(int)*(size_t) nowner,cudaMemcpyHostToDevice,st));
+  CUDA_TRY(cudaMemsetAsync(d_cnt,0,8*64*2,st));
+  if ((rc = fgb_owner_count_device(d_in,n,field_pos,field_bits,d_owner,nowner,world,d_cnt,st))) return rc;
+  CUDA_TRY(cudaMemcpyAsync(cnt,d_cnt,8*64,cudaMemcpyDeviceToHost,st));
+  CUDA_TRY(cudaStreamSynchronize(st));
+  base[0] = 0;
+  for (int w = 0; w < world; w++) base[w+1] = base[w] + cnt[w];
+  CUDA_TRY(cudaMemcpyAsync(d_cnt + 64,base,8*64,cudaMemcpyHostToDevice,st));
+  if ((rc = fgb_owner_scatter_device(d_in,n,field_pos,field_bits,d_owner,nowner,world,d_cnt + 64,d_out,st))) return rc;
+  CUDA_TRY(cudaStreamSynchronize(st));
   for (int w = 0; w <= world; w++) bounds[w] = (long long) base[w];
   return FGB_OK;
 }
 
-//  k-mer records grouped by the rank that owns their first four bases: owner256[b] for top byte b;
-//  d_out[bounds[w] .. bounds[w+1]) are the records of owner w (count + scatter: cheaper than the radix
-//  pass of fgb_records_group_by_top_byte when only the destination matters)
+//  seeds grouped by the rank that owns their A-contig: owner[r] for contig RANK r (the icont field)
+extern "C" int fgb_seeds_group_by_owner(const void *d_seeds, long long n, const int *bits, const int *owner,
+                                        int nrank_contigs, int world, void *d_out, long long *bounds,
+                                        void *stream)
+{ return group_by_owner(d_seeds,n,12 + bits[0] + bits[1] + bits[2],bits[3],owner,nrank_contigs,world,d_out,bounds,
+                        (cudaStream_t) stream); }
+
+//  k-mer records grouped by the rank that owns their first four bases: owner256[b] for top byte b
 extern "C" int fgb_records_group_by_owner(const void *d_recs, long long n, const int *owner256, int world,
                                           void *d_out, long long *bounds, void *stream)
-{ cudaStream_t st = (cudaStream_t) stream;
-  if (world < 1 || world > 64) return FGB_ERR_ARG;
-  for (int w = 0; w <= world; w++) bounds[w] = 0;
-  if (n <= 0) return FGB_OK;
-  int *d_owner = NULL; u64 *d_cnt = NULL;
-  int rc = FGB_OK;
-  u64 cnt[64], base[65];
-  if (fgb_dmalloc((void **) &d_owner,sizeof(int)*256,st) != cudaSuccess ||
-      fgb_dmalloc((void **) &d_cnt,8*64*2,st) != cudaSuccess) rc = FGB_ERR_CUDA;
-  if (!rc && (cudaMemcpyAsync(d_owner,owner256,sizeof(int)*256,cudaMemcpyHostToDevice,st) != cudaSuccess ||
-              cudaMemsetAsync(d_cnt,0,8*64*2,st) != cudaSuccess)) rc = FGB_ERR_CUDA;
-  if (!rc) rc = fgb_owner_count_device(d_recs,n,120,8,d_owner,256,world,d_cnt,st);
-  if (!rc && (cudaMemcpyAsync(cnt,d_cnt,8*64,cudaMemcpyDeviceToHost,st) != cudaSuccess ||
-              cudaStreamSynchronize(st) != cudaSuccess)) rc = FGB_ERR_CUDA;
-  if (!rc)
-    { base[0] = 0;
-      for (int w = 0; w < world; w++) base[w+1] = base[w] + cnt[w];
-      if (cudaMemcpyAsync(d_cnt + 64,base,8*64,cudaMemcpyHostToDevice,st) != cudaSuccess) rc = FGB_ERR_CUDA;
-    }
-  if (!rc) rc = fgb_owner_scatter_device(d_recs,n,120,8,d_owner,256,world,d_cnt + 64,d_out,st);
-  if (!rc && cudaStreamSynchronize(st) != cudaSuccess) rc = FGB_ERR_CUDA;
-  fgb_dfree(d_owner,st); fgb_dfree(d_cnt,st);
-  if (rc) return rc;
-  for (int w = 0; w <= world; w++) bounds[w] = (long long) base[w];
-  return FGB_OK;
-}
+{ return group_by_owner(d_recs,n,120,8,owner256,256,world,d_out,bounds,(cudaStream_t) stream); }
 
 //  sorted seed set over n unsorted device records (copied); bits as fgb_seeds_merge returns them
 extern "C" int fgb_seeds_from_records(const void *d_recs, long long n, const int *bits, long long amxpos,
@@ -770,9 +621,9 @@ extern "C" int fgb_seeds_from_records(const void *d_recs, long long n, const int
   L.key = 12 + L.anti + L.band + L.jc + L.ic + 1;
   if (L.key > 128) return FGB_ERR_LIMIT;
   rec128 *d_a = NULL;
+  dev_scope S(st); S.own(d_a);
   CUDA_TRY(fgb_dmalloc((void **) &d_a,sizeof(rec128)*(n+1),st));
-  if (n > 0 && cudaMemcpyAsync(d_a,d_recs,sizeof(rec128)*n,cudaMemcpyDeviceToDevice,st) != cudaSuccess)
-    { fgb_dfree(d_a,st); return FGB_ERR_CUDA; }
+  if (n > 0) CUDA_TRY(cudaMemcpyAsync(d_a,d_recs,sizeof(rec128)*n,cudaMemcpyDeviceToDevice,st));
   return seeds_sort_impl(d_a,n,L,amxpos,bmxpos,false,sumlen,0,out,st);
 }
 
@@ -788,6 +639,7 @@ extern "C" int fgb_seeds_download(const fgb_seeds *s, void *rec)
 extern "C" int fgb_sort128_host(void *recs, long long n, int byte_lo, int byte_hi, void *stream)
 { cudaStream_t st = (cudaStream_t) stream;
   rec128 *d_a = NULL, *d_b = NULL; void *d_tmp = NULL;
+  dev_scope S(st); S.own(d_a); S.own(d_b); S.own(d_tmp);
   long long tmpb = fgb_sort128_tmp_bytes(n);
   CUDA_TRY(fgb_dmalloc((void **) &d_a,sizeof(rec128)*(n+1),st));
   CUDA_TRY(fgb_dmalloc((void **) &d_b,sizeof(rec128)*(n+1),st));
@@ -797,7 +649,6 @@ extern "C" int fgb_sort128_host(void *recs, long long n, int byte_lo, int byte_h
   int rc = fgb_sort128_device(d_a,d_b,n,byte_lo,byte_hi,d_tmp,tmpb,&inb,st);
   if (!rc) CUDA_TRY(cudaMemcpyAsync(recs,inb ? d_b : d_a,sizeof(rec128)*n,cudaMemcpyDeviceToHost,st));
   CUDA_TRY(cudaStreamSynchronize(st));
-  fgb_dfree(d_a,st); fgb_dfree(d_b,st); fgb_dfree(d_tmp,st);
   return rc;
 }
 
@@ -832,77 +683,32 @@ struct fgb_run_stats
             us_gix, us_seeds, us_extend, us_filter, nkmers1_fwd,
             slow_cycles, slow_waves, paired_waves, pairings; };
 
-//  Merge + seed sort + extension + filter from prebuilt tables (x2 may have been assembled from
-//  shares built on several ranks).
-extern "C" int fgb_align_tables(const fgb_genome *A, const fgb_genome *B, const fgb_gix *x1,
-                                const fgb_gix *x2, const float *freqA,
-                                int freq, int chain_break, int chain_min, int align_min,
-                                double align_rate, fgb_alns **out, fgb_run_stats *stats, void *stream);
-
-static int align_tables_impl(const fgb_genome *A, const fgb_genome *B, fgb_gix *x1, fgb_gix *x2, bool own,
-                             const float *freqA, int freq, int chain_break, int chain_min, int align_min,
-                             double align_rate, fgb_alns **out, fgb_run_stats *stats, void *stream);
-
-//  Device-resident genomes in, final alignments out (the timed "step" of bench.py).
-extern "C" int fgb_align_resident(const fgb_genome *A, const fgb_genome *B, const float *freqA,
-                                  int freq, int chain_break, int chain_min, int align_min,
-                                  double align_rate, fgb_alns **out, fgb_run_stats *stats, void *stream)
-{ fgb_gix *x1 = NULL, *x2 = NULL;
-  int rc;
-  long long t0 = now_us();
-  //  adaptamer side: forward strand only, and only the table (the merge reads the OTHER table's index)
-  if ((rc = gix_build_range(A,0u,(1u << 24) | GIX_FWD_ONLY | GIX_NO_INDEX,&x1,stream))) return rc;
-  if ((rc = fgb_gix_build(B,&x2,stream))) { fgb_gix_free(x1); return rc; }
-  long long t1 = now_us();
-  //  the tables are this call's own: they go back to the allocator as soon as the merge has read them
-  //  (two tables + seeds + sort buffer of a multi-Gbp pair do not fit side by side)
-  rc = align_tables_impl(A,B,x1,x2,true,freqA,freq,chain_break,chain_min,align_min,align_rate,out,stats,stream);
-  if (stats) stats->us_gix = t1 - t0;
-  return rc;
-}
-
-extern "C" int fgb_align_tables(const fgb_genome *A, const fgb_genome *B, const fgb_gix *x1,
-                                const fgb_gix *x2, const float *freqA,
-                                int freq, int chain_break, int chain_min, int align_min,
-                                double align_rate, fgb_alns **out, fgb_run_stats *stats, void *stream)
-{ return align_tables_impl(A,B,(fgb_gix *) x1,(fgb_gix *) x2,false,freqA,freq,chain_break,chain_min,align_min,
-                           align_rate,out,stats,stream);
-}
-
-static int align_tables_impl(const fgb_genome *A, const fgb_genome *B, fgb_gix *x1, fgb_gix *x2, bool own,
-                             const float *freqA, int freq, int chain_break, int chain_min, int align_min,
-                             double align_rate, fgb_alns **out, fgb_run_stats *stats, void *stream)
-{ fgb_seeds *sd = NULL; fgb_overlaps *ov = NULL;
-  int rc;
-  long long t0 = now_us(), t1 = t0, t2, t3, t4;
-  const long long n1 = x1->n_both, n2 = x2->n;
-  { seed_bits L;
-    rec128 *d_a = NULL; long long n = 0, sumlen = 0, n1m = 0;
-    rc = seed_layout_of(x1,x2,A->maxlen,B->maxlen,&L);
-    if (!rc) rc = seeds_merge_impl(x1,x2,A->maxlen,B->maxlen,freq,false,L,&d_a,&n,&sumlen,&n1m,(cudaStream_t) stream);
-    if (own) { fgb_gix_free(x1); fgb_gix_free(x2); }
-    if (!rc) rc = seeds_sort_impl(d_a,n,L,A->maxlen,B->maxlen,false,sumlen,n1m,&sd,(cudaStream_t) stream);
-  }
-  if (rc) return rc;
-  const long long n1f = sd->n1_merged;
-  t2 = now_us();
+//  The tail of both whole-path calls: extension of the seeds (released here), redundancy filter, and
+//  the seed and overlap counters of *stats (nseeds, sumlen, nhits .. nraw, nseg .. extract_cycles,
+//  slow_cycles .. pairings).  Where not NULL: *t_extended = host clock when the extension is done,
+//  *ovl_bytes = bytes of raw records read back from the device.
+static int extend_and_filter(fgb_seeds *sd, const fgb_genome *A, const fgb_genome *B, const float *freqA,
+                             int chain_break, int chain_min, int align_min, double align_rate,
+                             fgb_alns **out, fgb_run_stats *stats, long long *t_extended, long long *ovl_bytes,
+                             void *stream)
+{ fgb_overlaps *ov = NULL;
   short *tables = (short *) malloc(65536*sizeof(short));
   int ave = 0;
   fgb_align_spec(1.-align_rate,freqA,tables,&ave);           // FastGA.c:3760
-  rc = fgb_extend(sd,A,B,chain_break,chain_min,align_min,align_rate,tables,ave,100,&ov,stream);
+  int rc = fgb_extend(sd,A,B,chain_break,chain_min,align_min,align_rate,tables,ave,100,&ov,stream);
   free(tables);
-  t3 = now_us();
-  long long nseeds = sd->n, sumlen = sd->sumlen;
-  int jb = sd->jc_bits, ib = sd->ic_bits;
+  if (t_extended) *t_extended = now_us();
+  const long long nseeds = sd->n, sumlen = sd->sumlen;
+  const int jb = sd->jc_bits, ib = sd->ic_bits;
   fgb_seeds_free(sd);
   if (rc) return rc;
+  owner<fgb_overlaps> own(ov,fgb_overlaps_free);
   rc = fgb_filter(ov,A->perm.data(),B->perm.data(),jb,ib,1,out);
-  t4 = now_us();
+  if (ovl_bytes) *ovl_bytes = fgb_overlaps_bytes(ov);
   if (stats)
-    { stats->us_gix = t1-t0; stats->us_seeds = t2-t1; stats->us_extend = t3-t2; stats->us_filter = t4-t3; unsigned long long c[16];
+    { unsigned long long c[16];
       fgb_overlaps_counters(ov,c);
-      stats->nkmers1 = n1; stats->nkmers2 = n2; stats->nseeds = nseeds; stats->sumlen = sumlen;
-      stats->nkmers1_fwd = n1f;
+      stats->nseeds = nseeds; stats->sumlen = sumlen;
       stats->nhits = (long long) c[0]; stats->nla = (long long) c[1]; stats->nwaves = (long long) c[2];
       stats->ncells = (long long) c[3]; stats->nraw = 0;
       stats->nseg = (long long) c[5]; stats->nwork = (long long) c[6];
@@ -910,11 +716,46 @@ static int align_tables_impl(const fgb_genome *A, const fgb_genome *B, fgb_gix *
       stats->extract_cycles = (long long) c[10];
       stats->slow_cycles = (long long) ((c[15] >> 40) << 12); stats->slow_waves = (long long) ((c[15] >> 16) & 0xffffff);
       stats->paired_waves = (long long) c[11]; stats->pairings = (long long) c[12];
-      stats->h2d_bytes = A->h2d_bytes + B->h2d_bytes + 65536*2;
-      stats->d2h_bytes = fgb_overlaps_bytes(ov) + 16 + 8*1024*2 + 64;
     }
-  fgb_overlaps_free(ov);
   return rc;
+}
+
+//  Device-resident genomes in, final alignments out (the timed "step" of bench.py).
+extern "C" int fgb_align_resident(const fgb_genome *A, const fgb_genome *B, const float *freqA,
+                                  int freq, int chain_break, int chain_min, int align_min,
+                                  double align_rate, fgb_alns **out, fgb_run_stats *stats, void *stream)
+{ cudaStream_t st = (cudaStream_t) stream;
+  fgb_gix *x1 = NULL, *x2 = NULL;
+  int rc;
+  long long t0 = now_us();
+  //  adaptamer side: forward strand only, and only the table (the merge reads the OTHER table's index)
+  if ((rc = gix_build(A,true,false,&x1,st))) return rc;
+  owner<fgb_gix> own1(x1,fgb_gix_free);
+  if ((rc = gix_build(B,false,true,&x2,st))) return rc;
+  owner<fgb_gix> own2(x2,fgb_gix_free);
+  long long t1 = now_us();
+  const long long n1 = x1->n_both, n2 = x2->n;
+  seed_bits L;
+  rec128 *d_a = NULL; long long n = 0, sumlen = 0, n1m = 0;
+  rc = seed_layout_of(x1,x2,A->maxlen,B->maxlen,&L);
+  if (!rc) rc = seeds_merge_impl(x1,x2,A->maxlen,B->maxlen,freq,false,L,&d_a,&n,&sumlen,&n1m,st);
+  //  the tables go back to the allocator as soon as the merge has read them (two tables + seeds +
+  //  sort buffer of a multi-Gbp pair do not fit side by side)
+  own1.reset(); own2.reset();
+  if (rc) return rc;
+  fgb_seeds *sd = NULL;
+  if ((rc = seeds_sort_impl(d_a,n,L,A->maxlen,B->maxlen,false,sumlen,n1m,&sd,st))) return rc;
+  long long t2 = now_us(), t3 = t2, ovl_bytes = 0;
+  rc = extend_and_filter(sd,A,B,freqA,chain_break,chain_min,align_min,align_rate,out,stats,&t3,&ovl_bytes,stream);
+  long long t4 = now_us();
+  if (rc) return rc;
+  if (stats)
+    { stats->us_gix = t1-t0; stats->us_seeds = t2-t1; stats->us_extend = t3-t2; stats->us_filter = t4-t3;
+      stats->nkmers1 = n1; stats->nkmers2 = n2; stats->nkmers1_fwd = n1m;
+      stats->h2d_bytes = A->h2d_bytes + B->h2d_bytes + 65536*2;
+      stats->d2h_bytes = ovl_bytes + 16 + 8*1024*2 + 64;
+    }
+  return FGB_OK;
 }
 
 //  The reference-facing call: host .bps images + contig tables in, alignments out; every
@@ -925,35 +766,20 @@ extern "C" int fgb_fastga_self(const unsigned char *bps, long long nb, int nc, c
                                const long long *boff, const float *freq4,
                                int freq, int chain_break, int chain_min, int align_min, double align_rate,
                                fgb_alns **out, fgb_run_stats *stats, void *stream)
-{ fgb_genome *A = NULL; fgb_gix *x = NULL; fgb_seeds *sd = NULL; fgb_overlaps *ov = NULL;
+{ fgb_genome *A = NULL; fgb_gix *x = NULL; fgb_seeds *sd = NULL;
   int rc;
   if ((rc = fgb_genome_create(bps,nb,nc,clen,boff,1,&A,stream))) return rc;
-  if ((rc = fgb_gix_build(A,&x,stream))) { fgb_genome_free(A); return rc; }
+  owner<fgb_genome> own(A,fgb_genome_free);
+  if ((rc = fgb_gix_build(A,&x,stream))) return rc;
   rc = fgb_seeds_find_self(x,A->maxlen,freq,&sd,stream);
-  long long n1 = x->n;
+  const long long n1 = x->n;
   fgb_gix_free(x);
-  if (rc) { fgb_genome_free(A); return rc; }
-  short *tables = (short *) malloc(65536*sizeof(short));
-  int ave = 0;
-  fgb_align_spec(1.-align_rate,freq4,tables,&ave);
-  rc = fgb_extend(sd,A,A,chain_break,chain_min,align_min,align_rate,tables,ave,100,&ov,stream);
-  free(tables);
-  long long nseeds = sd->n, sumlen = sd->sumlen;
-  int jb = sd->jc_bits, ib = sd->ic_bits;
-  fgb_seeds_free(sd);
-  if (rc) { fgb_genome_free(A); return rc; }
-  rc = fgb_filter(ov,A->perm.data(),A->perm.data(),jb,ib,1,out);
-  if (stats)
-    { memset(stats,0,sizeof(*stats));
-      unsigned long long c[16];
-      fgb_overlaps_counters(ov,c);
-      stats->nkmers1 = stats->nkmers2 = n1; stats->nseeds = nseeds; stats->sumlen = sumlen;
-      stats->nhits = (long long) c[0]; stats->nla = (long long) c[1]; stats->nwaves = (long long) c[2];
-      stats->ncells = (long long) c[3];
-    }
-  fgb_overlaps_free(ov);
-  fgb_genome_free(A);
-  return rc;
+  if (rc) return rc;
+  if (stats) memset(stats,0,sizeof(*stats));
+  rc = extend_and_filter(sd,A,A,freq4,chain_break,chain_min,align_min,align_rate,out,stats,NULL,NULL,stream);
+  if (rc) return rc;
+  if (stats) stats->nkmers1 = stats->nkmers2 = n1;
+  return FGB_OK;
 }
 
 extern "C" int fgb_fastga(const unsigned char *bpsA, long long nbA, int ncA, const long long *clenA,

@@ -4,6 +4,8 @@
 #include <stdint.h>
 #include <stdio.h>
 #include <stdlib.h>
+#include <memory>
+#include <vector>
 
 #define FGB_OK            0
 #define FGB_ERR_CUDA     -1   // a CUDA runtime call failed (message on stderr)
@@ -61,12 +63,25 @@ int fgb_dev_exclusive_scan_u32(unsigned *d_data, long long n, unsigned long long
                                void *d_tmp, long long tmp_bytes, cudaStream_t st);
 long long fgb_dev_scan_tmp_bytes(long long n);
 
-void fgb_timing_add(int which, float ms);     // 0 triples 1 extend 2 d2h 3 merge kernel
 void fgb_count_launch(int n);                 // kernels launched (bench.py gpu_launches)
 
 //  stream-ordered device allocation from a retained pool (no cudaMalloc/cudaFree stalls per step)
 cudaError_t fgb_dmalloc(void **p, size_t bytes, cudaStream_t st);
 void fgb_dfree(void *p, cudaStream_t st);
+
+//  Device blocks of a call go back on EVERY way out of it, error returns included: the pointer
+//  variables are registered once (declare the scope after them), whatever they hold when the scope
+//  ends is released, in registration order.  A block handed to a handle or to the caller is
+//  cleared from its variable first.
+struct dev_scope
+{ cudaStream_t st; std::vector<void **> slots;
+  explicit dev_scope(cudaStream_t s) : st(s) {}
+  template<class T> void own(T *&p) { slots.push_back((void **) &p); }
+  ~dev_scope() { for (void **s : slots) if (*s != NULL) { fgb_dfree(*s,st); *s = NULL; } }
+};
+
+//  A handle released by its free function unless handed out with release().
+template<class T> using owner = std::unique_ptr<T,void (*)(T *)>;
 
 //  TMA 1-D bulk copy global -> shared (cp.async.bulk, SASS UBLKCP) completed on an mbarrier.
 //  dst/src 16-byte aligned, bytes a multiple of 16.  One elected thread issues; every thread of

@@ -2326,17 +2326,6 @@ static void tr_mark(const char *what)
 static bool tr_on() { static int on = -1; if (on < 0) on = (getenv("FGB_TRACE") != NULL); return on != 0; }
 #define TR_SYNC(what) do { if (tr_on()) { cudaStreamSynchronize(st); tr_mark(what); } } while (0)
 
-struct ev_timer
-{ cudaEvent_t a, b; cudaStream_t st; int which;
-  ev_timer(int w, cudaStream_t s) : st(s), which(w)
-    { cudaEventCreate(&a); cudaEventCreate(&b); cudaEventRecord(a,st); }
-  ~ev_timer()
-    { cudaEventRecord(b,st); cudaEventSynchronize(b);
-      float ms = 0; cudaEventElapsedTime(&ms,a,b); fgb_timing_add(which,ms);
-      cudaEventDestroy(a); cudaEventDestroy(b);
-    }
-};
-
 //  tables: 2 x 32768 int16 (score, then table) and ave_path from New_Align_Spec's arithmetic,
 //  computed by the host caller (align.c:222-268 is float/double set-up, kept on the host).
 
@@ -2456,21 +2445,6 @@ extern "C" long long fgb_hit_groups_host(int nwork, const unsigned *hrange, cons
   return (long long) items.size();
 }
 
-//  Device blocks (and the result handle) of a call go back on EVERY way out of it, error returns included:
-//  the pointer variables are registered once, whatever they hold when the scope ends is released.
-struct dev_scope
-{ cudaStream_t st; std::vector<void **> slots;
-  explicit dev_scope(cudaStream_t s) : st(s) {}
-  template<class T> void own(T *&p) { slots.push_back((void **) &p); }
-  ~dev_scope() { for (void **s : slots) if (*s != NULL) { fgb_dfree(*s,st); *s = NULL; } }
-};
-struct ovl_scope
-{ fgb_overlaps *o;
-  explicit ovl_scope(fgb_overlaps *p) : o(p) {}
-  fgb_overlaps *release() { fgb_overlaps *p = o; o = NULL; return p; }
-  ~ovl_scope() { if (o != NULL) fgb_overlaps_free(o); }
-};
-
 extern "C" int fgb_extend(const fgb_seeds *S, const fgb_genome *A, const fgb_genome *B,
                           int chain_break, int chain_min, int align_min, double align_rate,
                           const short *tables, int ave_path, int tspace,
@@ -2478,9 +2452,8 @@ extern "C" int fgb_extend(const fgb_seeds *S, const fgb_genome *A, const fgb_gen
 { cudaStream_t st = (cudaStream_t) stream;
   if (A->d_rseq == NULL) return FGB_ERR_ARG;
   if (S->n >= 0xfffffff0ll) return FGB_ERR_LIMIT;
-  fgb_overlaps *O = new fgb_overlaps();
-  ovl_scope Oown(O);
-  dev_scope G(st);
+  owner<fgb_overlaps> Oown(new fgb_overlaps(),fgb_overlaps_free);
+  fgb_overlaps *O = Oown.get();
   long long n = S->n;
   tr_mark("extend: enter");
 
@@ -2505,8 +2478,18 @@ extern "C" int fgb_extend(const fgb_seeds *S, const fgb_genome *A, const fgb_gen
   u64 *d_counters = NULL, *d_total = NULL;
   unsigned *d_flag = NULL, *d_seg = NULL, *d_work = NULL, *d_misc = NULL, *d_failed = NULL;
   void *d_tmp = NULL;
+  ChunkPlan *d_plan = NULL; ChunkOut *d_couts = NULL; unsigned *d_first = NULL, *d_failed_w = NULL;
+  ChainHit *d_hits = NULL; uint2 *d_hrange = NULL;
+  //  hit groups (first launch): items in launch order, and for each the first hit of the NEXT group of
+  //  its triple (what its tube must not have reached for the groups to have been independent)
+  ExItem *d_items = NULL; long long *d_galast = NULL; int2 *d_tinfo = NULL;
+  unsigned char *d_out = NULL;
+  dev_scope G(st);
   G.own(d_tables); G.own(d_counters); G.own(d_total); G.own(d_flag); G.own(d_seg); G.own(d_work);
   G.own(d_misc); G.own(d_failed); G.own(d_tmp);
+  G.own(d_plan); G.own(d_couts); G.own(d_first); G.own(d_failed_w); G.own(d_hits); G.own(d_hrange);
+  G.own(d_items); G.own(d_galast); G.own(d_tinfo);
+  G.own(d_out);
   CUDA_TRY(fgb_dmalloc((void **) &d_tables,65536*sizeof(short),st));
   CUDA_TRY(cudaMemcpyAsync(d_tables,tables,65536*sizeof(short),cudaMemcpyHostToDevice,st));
   P.score = d_tables; P.table = d_tables + 32768;
@@ -2519,18 +2502,12 @@ extern "C" int fgb_extend(const fgb_seeds *S, const fgb_genome *A, const fgb_gen
 
   unsigned nseg = 0, nwork = 0;
   std::vector<unsigned> wsize; bool sizes_known = false;
-  ChunkPlan *d_plan = NULL; ChunkOut *d_couts = NULL; unsigned *d_first = NULL, *d_failed_w = NULL;
-  ChainHit *d_hits = NULL; uint2 *d_hrange = NULL; unsigned long long hit_cap = 0;
-  //  hit groups (first launch): items in launch order, and for each the first hit of the NEXT group of
-  //  its triple (what its tube must not have reached for the groups to have been independent)
-  ExItem *d_items = NULL; long long *d_galast = NULL; int2 *d_tinfo = NULL;
-  G.own(d_plan); G.own(d_couts); G.own(d_first); G.own(d_failed_w); G.own(d_hits); G.own(d_hrange);
-  G.own(d_items); G.own(d_galast); G.own(d_tinfo);
+  unsigned long long hit_cap = 0;
   std::vector<ExItem> items; std::vector<long long> nxt_alow, nxt_ahgh;
   std::vector<unsigned> hwork, hcount;                 // work triples; hits of each pre-scanned one
   unsigned long long hits_done = 0;                    // hits of the pre-scanned triples the first launch completed
   if (n > 0)
-    { ev_timer t(0,st);
+    { stage_timer t(&g_timings.triples_ms,st);
       long long tmpb = fgb_dev_scan_tmp_bytes(n);
       CUDA_TRY(fgb_dmalloc((void **) &d_flag,sizeof(unsigned)*(n+1),st));
       CUDA_TRY(fgb_dmalloc((void **) &d_tmp,tmpb,st));
@@ -2687,8 +2664,6 @@ extern "C" int fgb_extend(const fgb_seeds *S, const fgb_genome *A, const fgb_gen
   O->nseg = nseg; O->nwork = nwork;
   tr_mark("extend: triples+prefilter");
 
-  unsigned char *d_out = NULL;
-  G.own(d_out);
   u64 out_cap = 0, out_used = 0;
   if (nwork > 0)
     { int dev = 0, nsm = 148;
@@ -2723,58 +2698,57 @@ extern "C" int fgb_extend(const fgb_seeds *S, const fgb_genome *A, const fgb_gen
       dev_scope G2(st); G2.own(d_work2);
       u64 used_before = 0;
       for (int attempt = 0; nlist > 0; attempt++)
-        { Peb *d_cells = NULL; unsigned char *d_stage = NULL; unsigned char *d_big = NULL;
-          unsigned long long *d_wlog = NULL;
-          dev_scope L(st); L.own(d_cells); L.own(d_stage); L.own(d_big); L.own(d_wlog);
-          CUDA_TRY(fgb_dmalloc((void **) &d_cells,sizeof(Peb)*cells_per_warp*nwarps,st));
-          CUDA_TRY(fgb_dmalloc((void **) &d_stage,2ll*stage_bytes*nwarps,st));
-          if (d_out == NULL) CUDA_TRY(fgb_dmalloc((void **) &d_out,out_cap,st));
-          P.cells = d_cells; P.cells_per_warp = cells_per_warp;
-          P.stage = d_stage; P.stage_bytes = stage_bytes;
-          P.out = d_out; P.out_cap = out_cap;
-          P.work = d_list; P.nwork = (int) nlist;
-          P.items = use_items ? d_items : NULL; P.galast = d_galast; P.attempt = attempt;
-          if (attempt > 0)                                     // retries: wide-band kernel, state in HBM
-            { CUDA_TRY(fgb_dmalloc((void **) &d_big,(size_t) nwarps * WSTATE_BYTES(EX_WBIG),st));
-              P.bigstate = d_big;
+        { unsigned misc[12];
+          { Peb *d_cells = NULL; unsigned char *d_stage = NULL; unsigned char *d_big = NULL;
+            unsigned long long *d_wlog = NULL;
+            dev_scope L(st); L.own(d_wlog); L.own(d_cells); L.own(d_stage); L.own(d_big);    // arenas of this launch
+            CUDA_TRY(fgb_dmalloc((void **) &d_cells,sizeof(Peb)*cells_per_warp*nwarps,st));
+            CUDA_TRY(fgb_dmalloc((void **) &d_stage,2ll*stage_bytes*nwarps,st));
+            if (d_out == NULL) CUDA_TRY(fgb_dmalloc((void **) &d_out,out_cap,st));
+            P.cells = d_cells; P.cells_per_warp = cells_per_warp;
+            P.stage = d_stage; P.stage_bytes = stage_bytes;
+            P.out = d_out; P.out_cap = out_cap;
+            P.work = d_list; P.nwork = (int) nlist;
+            P.items = use_items ? d_items : NULL; P.galast = d_galast; P.attempt = attempt;
+            if (attempt > 0)                                     // retries: wide-band kernel, state in HBM
+              { CUDA_TRY(fgb_dmalloc((void **) &d_big,(size_t) nwarps * WSTATE_BYTES(EX_WBIG),st));
+                P.bigstate = d_big;
+              }
+            tr_mark("extend: arenas allocated");
+            if (attempt == 0 && getenv("FGB_WLOG") != NULL)
+              { CUDA_TRY(fgb_dmalloc((void **) &d_wlog,32ull*(nlist+1),st));
+                CUDA_TRY(cudaMemsetAsync(d_wlog,0,32ull*(nlist+1),st));
+              }
+            P.wlog = d_wlog;
+            CUDA_TRY(cudaMemsetAsync(d_misc+1,0,8,st));          // queue, nfailed
+            CUDA_TRY(cudaMemsetAsync(d_misc+10,0,4,st));         // reasons of this attempt's failures
+            { stage_timer t(&g_timings.extend_ms,st);
+              if (attempt == 0)
+                extend_kernel<EX_W><<<(unsigned) nblocks,EX_WARPS*32,smem,st>>>(P);
+              else
+                extend_kernel<EX_WBIG><<<(unsigned) nblocks,EX_WARPS*32,smem_big,st>>>(P);
             }
-          tr_mark("extend: arenas allocated");
-          if (attempt == 0 && getenv("FGB_WLOG") != NULL)
-            { CUDA_TRY(fgb_dmalloc((void **) &d_wlog,32ull*(nlist+1),st));
-              CUDA_TRY(cudaMemsetAsync(d_wlog,0,32ull*(nlist+1),st));
-            }
-          P.wlog = d_wlog;
-          CUDA_TRY(cudaMemsetAsync(d_misc+1,0,8,st));          // queue, nfailed
-          CUDA_TRY(cudaMemsetAsync(d_misc+10,0,4,st));         // reasons of this attempt's failures
-          { ev_timer t(1,st);
-            if (attempt == 0)
-              extend_kernel<EX_W><<<(unsigned) nblocks,EX_WARPS*32,smem,st>>>(P);
-            else
-              extend_kernel<EX_WBIG><<<(unsigned) nblocks,EX_WARPS*32,smem_big,st>>>(P);
+            g_timings.extend_launches += 1;
+            fgb_count_launch(1);
+            CUDA_TRY(cudaGetLastError());
+            CUDA_TRY(cudaMemcpyAsync(misc,d_misc,48,cudaMemcpyDeviceToHost,st));
+            CUDA_TRY(cudaStreamSynchronize(st));
+            tr_mark("extend: kernel done");
+            if (d_wlog != NULL)
+              { std::vector<unsigned long long> lg(4ull*nlist);
+                CUDA_TRY(cudaMemcpy(lg.data(),d_wlog,32ull*nlist,cudaMemcpyDeviceToHost));
+                FILE *f = fopen(getenv("FGB_WLOG"),"w");
+                if (f != NULL)
+                  { for (unsigned q = 0; q < nlist; q++)
+                      fprintf(f,"%u %llu %llu %llu %llu %llu %llu %llu %u %u %u\n",q,lg[4*q] >> 32,lg[4*q] & 0xffffffffull,
+                              lg[4*q+1] >> 24,(lg[4*q+1] >> 8) & 0xffff,lg[4*q+1] & 0xff,lg[4*q+2],lg[4*q+3],
+                              (P.items != NULL ? (items[q].w < wsize.size() ? wsize[items[q].w] : 0u)
+                                               : (q < wsize.size() ? wsize[q] : 0u)),
+                              P.items != NULL ? (items[q].hn & 0x7fffffffu) : 0u,P.items != NULL ? items[q].g : 0u);
+                    fclose(f);
+                  }
+              }
           }
-          fgb_count_launch(1);
-          CUDA_TRY(cudaGetLastError());
-          unsigned misc[12];
-          CUDA_TRY(cudaMemcpyAsync(misc,d_misc,48,cudaMemcpyDeviceToHost,st));
-          CUDA_TRY(cudaStreamSynchronize(st));
-          tr_mark("extend: kernel done");
-          if (d_wlog != NULL)
-            { std::vector<unsigned long long> lg(4ull*nlist);
-              CUDA_TRY(cudaMemcpy(lg.data(),d_wlog,32ull*nlist,cudaMemcpyDeviceToHost));
-              FILE *f = fopen(getenv("FGB_WLOG"),"w");
-              if (f != NULL)
-                { for (unsigned q = 0; q < nlist; q++)
-                    fprintf(f,"%u %llu %llu %llu %llu %llu %llu %llu %u %u %u\n",q,lg[4*q] >> 32,lg[4*q] & 0xffffffffull,
-                            lg[4*q+1] >> 24,(lg[4*q+1] >> 8) & 0xffff,lg[4*q+1] & 0xff,lg[4*q+2],lg[4*q+3],
-                            (P.items != NULL ? (items[q].w < wsize.size() ? wsize[items[q].w] : 0u)
-                                             : (q < wsize.size() ? wsize[q] : 0u)),
-                            P.items != NULL ? (items[q].hn & 0x7fffffffu) : 0u,P.items != NULL ? items[q].g : 0u);
-                  fclose(f);
-                }
-              fgb_dfree(d_wlog,st); d_wlog = NULL;
-            }
-          fgb_dfree(d_cells,st); fgb_dfree(d_stage,st); fgb_dfree(d_big,st);
-          d_cells = NULL; d_stage = NULL; d_big = NULL;
           out_used = ((u64) misc[5] << 32) | misc[4];
           unsigned nfailed = misc[2];
           if (out_used > out_cap)
@@ -2826,7 +2800,7 @@ extern "C" int fgb_extend(const fgb_seeds *S, const fgb_genome *A, const fgb_gen
           //  rerun only the failed triples (whole, hit after hit) with larger arenas on fewer warps; the
           //  records of their earlier launches are dropped by the host below.
           for (size_t q = 0; q < f.size(); q++) todo.push_back(std::make_pair(f[q],attempt + 1));
-          if (d_work2 == NULL) CUDA_TRY(cudaMalloc(&d_work2,sizeof(unsigned)*2*(nwork+1)));
+          if (d_work2 == NULL) CUDA_TRY(fgb_dmalloc((void **) &d_work2,sizeof(unsigned)*2*(nwork+1),st));
           CUDA_TRY(cudaMemcpy(d_work2,f.data(),sizeof(unsigned)*nfailed,cudaMemcpyHostToDevice));
           CUDA_TRY(cudaMemcpy(d_work2 + nwork + 1,fw.data(),sizeof(unsigned)*nfailed,cudaMemcpyHostToDevice));
           P.widx = d_work2 + nwork + 1;
@@ -2841,7 +2815,6 @@ extern "C" int fgb_extend(const fgb_seeds *S, const fgb_genome *A, const fgb_gen
           nblocks = nb2 < maxb ? nb2 : maxb;
           nwarps = nblocks * EX_WARPS;
         }
-      fgb_dfree(d_work2,st); d_work2 = NULL;
 
       //  bring the records back and drop partial output of triples that were re-run
       O->nbytes = (long long) out_used;
@@ -2855,7 +2828,7 @@ extern "C" int fgb_extend(const fgb_seeds *S, const fgb_genome *A, const fgb_gen
         }
       O->h_buf = (unsigned char *) malloc(out_used + 64);
       O->pinned = false;
-      { ev_timer t(2,st);
+      { stage_timer t(&g_timings.d2h_ms,st);
         CUDA_TRY(cudaMemcpyAsync(pin,d_out,out_used,cudaMemcpyDeviceToHost,st));
       }
       CUDA_TRY(cudaStreamSynchronize(st));
@@ -2943,22 +2916,22 @@ extern "C" int fgb_local_alignments(const fgb_genome *A, const fgb_genome *B, lo
   const size_t smem = (size_t) EX_WARPS * STATE_BYTES;
   short *d_tables = NULL; la_job *d_jobs = NULL; int *d_status = NULL; unsigned *d_misc = NULL;
   Peb *d_cells = NULL; unsigned char *d_stage = NULL, *d_out = NULL;
+  dev_scope S(st); S.own(d_tables); S.own(d_jobs); S.own(d_status); S.own(d_misc); S.own(d_cells); S.own(d_stage);
+  S.own(d_out);
   std::vector<unsigned char> h;
   std::vector<int> hs(n);
   u64 out_cap = (u64) n * 256 + (u64) traces_cap + (1ull << 20), out_used = 0;
-  int rc = FGB_OK;
-#define LA_TRY(call) do { if ((call) != cudaSuccess) { rc = FGB_ERR_CUDA; goto done; } } while (0)
-  LA_TRY(cudaFuncSetAttribute(la_batch_kernel,cudaFuncAttributeMaxDynamicSharedMemorySize,(int) smem));
-  LA_TRY(fgb_dmalloc((void **) &d_tables,65536*sizeof(short),st));
-  LA_TRY(fgb_dmalloc((void **) &d_jobs,sizeof(la_job)*(size_t) n,st));
-  LA_TRY(fgb_dmalloc((void **) &d_status,sizeof(int)*(size_t) n,st));
-  LA_TRY(fgb_dmalloc((void **) &d_misc,64,st));
-  LA_TRY(fgb_dmalloc((void **) &d_cells,sizeof(Peb)*cells_per_warp*nwarps,st));
-  LA_TRY(fgb_dmalloc((void **) &d_stage,2ll*stage_bytes*nwarps,st));
-  LA_TRY(fgb_dmalloc((void **) &d_out,out_cap,st));
-  LA_TRY(cudaMemcpyAsync(d_tables,tables,65536*sizeof(short),cudaMemcpyHostToDevice,st));
-  LA_TRY(cudaMemcpyAsync(d_jobs,jobs,sizeof(la_job)*(size_t) n,cudaMemcpyHostToDevice,st));
-  LA_TRY(cudaMemsetAsync(d_misc,0,64,st));
+  CUDA_TRY(cudaFuncSetAttribute(la_batch_kernel,cudaFuncAttributeMaxDynamicSharedMemorySize,(int) smem));
+  CUDA_TRY(fgb_dmalloc((void **) &d_tables,65536*sizeof(short),st));
+  CUDA_TRY(fgb_dmalloc((void **) &d_jobs,sizeof(la_job)*(size_t) n,st));
+  CUDA_TRY(fgb_dmalloc((void **) &d_status,sizeof(int)*(size_t) n,st));
+  CUDA_TRY(fgb_dmalloc((void **) &d_misc,64,st));
+  CUDA_TRY(fgb_dmalloc((void **) &d_cells,sizeof(Peb)*cells_per_warp*nwarps,st));
+  CUDA_TRY(fgb_dmalloc((void **) &d_stage,2ll*stage_bytes*nwarps,st));
+  CUDA_TRY(fgb_dmalloc((void **) &d_out,out_cap,st));
+  CUDA_TRY(cudaMemcpyAsync(d_tables,tables,65536*sizeof(short),cudaMemcpyHostToDevice,st));
+  CUDA_TRY(cudaMemcpyAsync(d_jobs,jobs,sizeof(la_job)*(size_t) n,cudaMemcpyHostToDevice,st));
+  CUDA_TRY(cudaMemsetAsync(d_misc,0,64,st));
   P.score = d_tables; P.table = d_tables + 32768;
   P.cells = d_cells; P.cells_per_warp = cells_per_warp;
   P.stage = d_stage; P.stage_bytes = stage_bytes;
@@ -2966,13 +2939,13 @@ extern "C" int fgb_local_alignments(const fgb_genome *A, const fgb_genome *B, lo
   P.queue = d_misc + 1;
   la_batch_kernel<<<(unsigned) nblocks,EX_WARPS*32,smem,st>>>(P,d_jobs,(int) n,d_status);
   fgb_count_launch(1);
-  LA_TRY(cudaGetLastError());
-  LA_TRY(cudaMemcpyAsync(&out_used,d_misc + 4,8,cudaMemcpyDeviceToHost,st));
-  LA_TRY(cudaMemcpyAsync(hs.data(),d_status,sizeof(int)*(size_t) n,cudaMemcpyDeviceToHost,st));
-  LA_TRY(cudaStreamSynchronize(st));
-  if (out_used > out_cap) { rc = FGB_ERR_OVERFLOW; goto done; }
+  CUDA_TRY(cudaGetLastError());
+  CUDA_TRY(cudaMemcpyAsync(&out_used,d_misc + 4,8,cudaMemcpyDeviceToHost,st));
+  CUDA_TRY(cudaMemcpyAsync(hs.data(),d_status,sizeof(int)*(size_t) n,cudaMemcpyDeviceToHost,st));
+  CUDA_TRY(cudaStreamSynchronize(st));
+  if (out_used > out_cap) return FGB_ERR_OVERFLOW;
   h.resize((size_t) out_used + 64);
-  LA_TRY(cudaMemcpy(h.data(),d_out,out_used,cudaMemcpyDeviceToHost));
+  CUDA_TRY(cudaMemcpy(h.data(),d_out,out_used,cudaMemcpyDeviceToHost));
   { long long used = 0;
     for (long long i = 0; i < n; i++)
       { int *p = paths + 7*i;
@@ -2990,13 +2963,9 @@ extern "C" int fgb_local_alignments(const fgb_genome *A, const fgb_genome *B, lo
         off += OUT_HDR + ((r[8] + 7) & ~7);
       }
     *traces_used = used;
-    if (used > traces_cap) rc = FGB_ERR_OVERFLOW;
+    if (used > traces_cap) return FGB_ERR_OVERFLOW;
   }
-done:
-#undef LA_TRY
-  fgb_dfree(d_tables,st); fgb_dfree(d_jobs,st); fgb_dfree(d_status,st); fgb_dfree(d_misc,st);
-  fgb_dfree(d_cells,st); fgb_dfree(d_stage,st); fgb_dfree(d_out,st);
-  return rc;
+  return FGB_OK;
 }
 
 extern "C" long long fgb_overlaps_count(const fgb_overlaps *o) { return o->nrec; }

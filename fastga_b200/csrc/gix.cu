@@ -182,16 +182,12 @@ syncmer_kernel(const u64 *__restrict__ seq, const long long *__restrict__ clen,
                const int *__restrict__ tile_contig, const int *__restrict__ tile_start,
                unsigned *__restrict__ tile_count,       // EMIT=0: out counts; EMIT=1: in offsets
                unsigned long long *__restrict__ buck1024,
-               rec128 *__restrict__ out, unsigned plo, unsigned phi_flags)
+               rec128 *__restrict__ out, int fwd_only)
 { __shared__ u64 sw[SC_WORDS+1];
   __shared__ unsigned char tn[256], tc[256];
   __shared__ unsigned wsum[SC_THREADS/32];
   __shared__ unsigned hist[1024];
 
-  //  bit 31 of phi_flags: forward-strand entries only (the table is only ever the adaptamer side
-  //  of a merge, where reverse entries never seed, FastGA.c:921-928)
-  const unsigned phi = phi_flags & 0x7fffffffu;
-  const bool fwd_only = (phi_flags >> 31) != 0;
   int tid = threadIdx.x;
   int c   = tile_contig[blockIdx.x];
   int t0  = tile_start[blockIdx.x];
@@ -225,22 +221,8 @@ syncmer_kernel(const u64 *__restrict__ seq, const long long *__restrict__ clen,
     int rl = 28 - p;                           // rev ok for i >= rl
     if (rl > 0) rmask = (rl >= SC_PPT) ? 0 : (rmask & ~((1u << rl) - 1));
   }
-  if (plo != 0 || phi != (1u << 24))               // keep only k-mers whose 12-base prefix is in [plo,phi)
-    { unsigned m = fmask | rmask;
-      while (m)
-        { int i = __ffs(m)-1;
-          m &= m-1;
-          if (fmask >> i & 1)
-            { unsigned pf = (unsigned) (rev2(sm_bases64(sw,sb+i)) >> 40);
-              if (pf < plo || pf >= phi) fmask &= ~(1u << i);
-            }
-          if (rmask >> i & 1)
-            { u64 e0 = sm_bases64(sw,sb+i-28), e1 = sm_bases64(sw,sb+i+4) & 0xffffull;
-              unsigned pr = (unsigned) ((~((e1 << 48) | (e0 >> 16))) >> 40);
-              if (pr < plo || pr >= phi) rmask &= ~(1u << i);
-            }
-        }
-    }
+  //  fwd_only: forward-strand entries only (the table is only ever the adaptamer side of a merge,
+  //  where reverse entries never seed, FastGA.c:921-928)
   unsigned rdropped = 0;                       // reverse entries a forward-only table leaves out
   if (fwd_only) { rdropped = __popc(rmask); rmask = 0; }
   unsigned cnt = __popc(fmask) + __popc(rmask);
@@ -458,7 +440,7 @@ extern "C" int fgb_syncmer_count_device(const void *d_seq, const long long *d_cl
                                         const int *d_tile_contig, const int *d_tile_start, int ntiles,
                                         unsigned *d_tile_count, unsigned long long *d_buck1024,
                                         unsigned long long *d_total, void *d_tmp, long long tmp_bytes,
-                                        unsigned plo, unsigned phi, void *stream)
+                                        int fwd_only, void *stream)
 { cudaStream_t st = (cudaStream_t) stream;
   int rc = init_tables();
   if (rc) return rc;
@@ -466,7 +448,7 @@ extern "C" int fgb_syncmer_count_device(const void *d_seq, const long long *d_cl
   if (ntiles > 0)
     syncmer_kernel<0><<<ntiles,SC_THREADS,0,st>>>((const u64 *) d_seq,d_clen,d_woff,d_crank,
                                                    d_tile_contig,d_tile_start,d_tile_count,
-                                                   d_buck1024,NULL,plo,phi);
+                                                   d_buck1024,NULL,fwd_only);
   fgb_count_launch(1);
   CUDA_TRY(cudaGetLastError());
   return fgb_dev_exclusive_scan_u32(d_tile_count,ntiles,d_total,d_tmp,tmp_bytes,st);
@@ -475,13 +457,13 @@ extern "C" int fgb_syncmer_count_device(const void *d_seq, const long long *d_cl
 extern "C" int fgb_syncmer_emit_device(const void *d_seq, const long long *d_clen,
                                        const long long *d_woff, const int *d_crank,
                                        const int *d_tile_contig, const int *d_tile_start, int ntiles,
-                                       unsigned *d_tile_offset, void *d_records, unsigned plo,
-                                       unsigned phi, void *stream)
+                                       unsigned *d_tile_offset, void *d_records, int fwd_only,
+                                       void *stream)
 { cudaStream_t st = (cudaStream_t) stream;
   if (ntiles > 0)
     syncmer_kernel<1><<<ntiles,SC_THREADS,0,st>>>((const u64 *) d_seq,d_clen,d_woff,d_crank,
                                                    d_tile_contig,d_tile_start,d_tile_offset,
-                                                   NULL,(rec128 *) d_records,plo,phi);
+                                                   NULL,(rec128 *) d_records,fwd_only);
   fgb_count_launch(1);
   CUDA_TRY(cudaGetLastError());
   return FGB_OK;

@@ -1,11 +1,28 @@
-// Opaque handle layouts behind the C-ABI (include/fastga_b200.h only forward-declares them).
+// Opaque handle layouts behind the C-ABI (include/fastga_b200.h only forward-declares them), and
+// the per-stage device timings.
 #pragma once
+#include <cuda_runtime.h>
 #include <vector>
 
 struct fgb_timings            // device milliseconds per stage (CUDA events on the call's stream)
 { float h2d_ms, stage_ms, scan_ms, ksort_ms, index_ms, merge_ms, ssort_ms, triples_ms, extend_ms,
         d2h_ms, filter_ms;
   int   merge_launches, extend_launches, launches;
+};
+
+extern fgb_timings g_timings;             // fgb_timings_get / fgb_timings_reset
+
+//  Adds the device time of the work issued on `s` during its lifetime to *d (one of the g_timings
+//  fields); waits for that work when it ends.
+struct stage_timer
+{ cudaEvent_t a, b; cudaStream_t st; float *dst;
+  stage_timer(float *d, cudaStream_t s) : st(s), dst(d)
+    { cudaEventCreate(&a); cudaEventCreate(&b); cudaEventRecord(a,st); }
+  ~stage_timer()
+    { cudaEventRecord(b,st); cudaEventSynchronize(b);
+      float ms = 0; cudaEventElapsedTime(&ms,a,b); *dst += ms;
+      cudaEventDestroy(a); cudaEventDestroy(b);
+    }
 };
 
 struct fgb_genome

@@ -20,6 +20,7 @@
 // memory, then every thread builds one 128-bit seed record per step and the stores of the CTA are
 // one contiguous run reserved with ONE atomic.
 #include "common.cuh"
+#include "handles.h"
 
 typedef unsigned long long u64;
 
@@ -460,25 +461,22 @@ extern "C" int fgb_forward_view_device(const void *d_T, long long n, void *d_out
   *h_nfwd = 0;
   if (n <= 0) return FGB_OK;
   unsigned *d_flag = NULL; void *d_tmp = NULL; unsigned long long *d_total = NULL;
+  dev_scope S(st); S.own(d_flag); S.own(d_tmp); S.own(d_total);
   long long tmpb = fgb_dev_scan_tmp_bytes(n);
-  cudaError_t e;
-  if ((e = fgb_dmalloc((void **) &d_flag,sizeof(unsigned)*(n+1),st)) != cudaSuccess ||
-      (e = fgb_dmalloc(&d_tmp,tmpb,st)) != cudaSuccess ||
-      (e = fgb_dmalloc((void **) &d_total,8,st)) != cudaSuccess)
-    { fgb_dfree(d_flag,st); fgb_dfree(d_tmp,st); fgb_dfree(d_total,st); return FGB_ERR_CUDA; }
+  CUDA_TRY(fgb_dmalloc((void **) &d_flag,sizeof(unsigned)*(n+1),st));
+  CUDA_TRY(fgb_dmalloc(&d_tmp,tmpb,st));
+  CUDA_TRY(fgb_dmalloc((void **) &d_total,8,st));
   int nb = (int) ((n + 255) / 256);
   fwd_flag_kernel<<<nb,256,0,st>>>((const rec128 *) d_T,n,d_flag);
   int rc = fgb_dev_exclusive_scan_u32(d_flag,n,d_total,d_tmp,tmpb,st);
+  if (rc) return rc;
+  fwd_scatter_kernel<<<nb,256,0,st>>>((const rec128 *) d_T,n,d_flag,(rec128 *) d_out);
+  fgb_count_launch(2);
   unsigned long long tot = 0;
-  if (!rc)
-    { fwd_scatter_kernel<<<nb,256,0,st>>>((const rec128 *) d_T,n,d_flag,(rec128 *) d_out);
-      fgb_count_launch(2);
-      if (cudaMemcpyAsync(&tot,d_total,8,cudaMemcpyDeviceToHost,st) != cudaSuccess ||
-          cudaStreamSynchronize(st) != cudaSuccess) rc = FGB_ERR_CUDA;
-    }
-  fgb_dfree(d_flag,st); fgb_dfree(d_tmp,st); fgb_dfree(d_total,st);
+  CUDA_TRY(cudaMemcpyAsync(&tot,d_total,8,cudaMemcpyDeviceToHost,st));
+  CUDA_TRY(cudaStreamSynchronize(st));
   *h_nfwd = (long long) tot;
-  return rc;
+  return FGB_OK;
 }
 
 /***********************************************************************************************
@@ -611,17 +609,12 @@ static int merge_launch(const rec128 *T1, unsigned n1, const rec128 *T2, const u
   unsigned nb = (unsigned) (((unsigned long long) n1 + TILE - 1) / TILE);
   uint4 *d_rng = NULL;
   CUDA_TRY(fgb_dmalloc((void **) &d_rng,sizeof(uint4)*(size_t) nb,st));
-  cudaEvent_t ea, eb;
-  cudaEventCreate(&ea); cudaEventCreate(&eb);
-  cudaEventRecord(ea,st);
-  merge_ranges_kernel<<<(nb + 255)/256,256,0,st>>>(T1,n1,pstart2,(unsigned) TILE,nb,d_rng);
-  adaptamer_merge_kernel<TILE><<<nb,MG_THREADS,smem,st>>>(T1,n1,T2,pstart2,adj2,d_rng,freq,K,seeds,capacity,counters);
-  cudaEventRecord(eb,st);
-  cudaEventSynchronize(eb);
-  float ms = 0; cudaEventElapsedTime(&ms,ea,eb);
-  fgb_timing_add(3,ms);
+  { stage_timer t(&g_timings.merge_ms,st);
+    merge_ranges_kernel<<<(nb + 255)/256,256,0,st>>>(T1,n1,pstart2,(unsigned) TILE,nb,d_rng);
+    adaptamer_merge_kernel<TILE><<<nb,MG_THREADS,smem,st>>>(T1,n1,T2,pstart2,adj2,d_rng,freq,K,seeds,capacity,counters);
+  }
+  g_timings.merge_launches += 1;
   fgb_count_launch(2);
-  cudaEventDestroy(ea); cudaEventDestroy(eb);
   fgb_dfree(d_rng,st);
   return FGB_OK;
 }

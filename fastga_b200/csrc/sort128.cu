@@ -341,15 +341,6 @@ __global__ void kmer_bins_kernel(const rec128 *__restrict__ tab, long long n, in
   for (long long p = lo+1; p <= hi; p++) bin_start[p] = (unsigned) i;
 }
 
-//  bin_start[p], p = 0..65536, for bins = hi >> binshift (host-callable)
-extern "C" int fgb_kmer_bins_device(const void *d_tab, long long n, int binshift, unsigned *d_bins, void *stream)
-{ int nb = (int) ((n + 1 + 255) / 256);
-  kmer_bins_kernel<<<nb,256,0,(cudaStream_t) stream>>>((const rec128 *) d_tab,n,binshift,0ull,d_bins,65536ll);
-  fgb_count_launch(1);
-  CUDA_TRY(cudaGetLastError());
-  return FGB_OK;
-}
-
 //  One CTA sorts one group (<= BK_CAP records of <= BK_SPAN consecutive bins) by the full 128-bit
 //  value.  Fast path: a counting split on the next 10 key bits (shared-memory atomics) leaves
 //  sub-bins of one or two records, and every record finds its place by comparing itself with its
@@ -521,7 +512,7 @@ static const size_t BUCKET_SMEM = BK_CAP*sizeof(rec128) + (BK_NSUB + 32 + 256 + 
 //  boundaries come to the host to pack the groups).
 
 //  [plo,phi): the range of 12-base prefixes the records come from (the whole space, or one
-//  rank's share of a cooperatively built table).  The 65536 bins always tile THAT range, so a share
+//  rank's slice of a k-mer-space sharded table).  The 65536 bins always tile THAT range, so a share
 //  is binned as finely as a whole table of the same size (bins of 16 + log2(2^24/range) top bits;
 //  one more partition pass when that exceeds two bytes).
 
@@ -557,6 +548,8 @@ extern "C" int fgb_kmer_sort_range_device(void *d_a, void *d_b, long long n, uns
     }
 
   unsigned *d_bins = NULL;
+  uint2 *d_groups = NULL;
+  dev_scope S(st); S.own(d_bins); S.own(d_groups);
   CUDA_TRY(fgb_dmalloc((void **) &d_bins,sizeof(unsigned)*(size_t) (nbins+1),st));
   { int nb = (int) ((n + 1 + 255) / 256);
     kmer_bins_kernel<<<nb,256,0,st>>>(src,n,binshift,base,d_bins,nbins);
@@ -586,7 +579,6 @@ extern "C" int fgb_kmer_sort_range_device(void *d_a, void *d_b, long long n, uns
     if (gc) groups.push_back(make_uint2(gs,gc));
   }
 
-  uint2 *d_groups = NULL;
   if (!groups.empty())
     { CUDA_TRY(fgb_dmalloc((void **) &d_groups,sizeof(uint2)*groups.size(),st));
       CUDA_TRY(cudaMemcpyAsync(d_groups,groups.data(),sizeof(uint2)*groups.size(),cudaMemcpyHostToDevice,st));
@@ -599,6 +591,7 @@ extern "C" int fgb_kmer_sort_range_device(void *d_a, void *d_b, long long n, uns
       opre.push_back(ototal);
       std::vector<unsigned> cfrom(opre.begin(),opre.end()-1);            // position in the compact array
       rec128 *d_c1 = NULL, *d_c2 = NULL; void *d_ctmp = NULL; unsigned *d_seg = NULL;
+      dev_scope C(st); C.own(d_c1); C.own(d_c2); C.own(d_ctmp); C.own(d_seg);
       long long ctb = fgb_sort128_tmp_bytes(ototal);
       CUDA_TRY(fgb_dmalloc((void **) &d_c1,sizeof(rec128)*((size_t) ototal+1),st));
       CUDA_TRY(fgb_dmalloc((void **) &d_c2,sizeof(rec128)*((size_t) ototal+1),st));
@@ -616,17 +609,11 @@ extern "C" int fgb_kmer_sort_range_device(void *d_a, void *d_b, long long n, uns
       fgb_count_launch(2);
       CUDA_TRY(cudaGetLastError());
       CUDA_TRY(cudaStreamSynchronize(st));                // the staging vectors above must outlive the copies
-      fgb_dfree(d_c1,st); fgb_dfree(d_c2,st); fgb_dfree(d_ctmp,st); fgb_dfree(d_seg,st);
     }
   CUDA_TRY(cudaStreamSynchronize(st));
-  fgb_dfree(d_bins,st); if (d_groups) fgb_dfree(d_groups,st);
   *result_in_b = inb ^ 1;
   return FGB_OK;
 }
-
-extern "C" int fgb_kmer_sort_device(void *d_a, void *d_b, long long n, void *d_tmp, long long tmp_bytes,
-                                    int *result_in_b, void *stream)
-{ return fgb_kmer_sort_range_device(d_a,d_b,n,0,1u << 24,d_tmp,tmp_bytes,result_in_b,stream); }
 
 /***********************************************************************************************
  *  Generic exclusive scan of a u32 array (reduce / scan-of-sums / downsweep), used for stream

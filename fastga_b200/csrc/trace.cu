@@ -159,11 +159,12 @@ extern "C" int fgb_compute_trace_pts(const fgb_genome *A, const fgb_genome *B, l
                                      fgb_scripts **out, void *stream)
 { cudaStream_t st = (cudaStream_t) stream;
   if (n < 0 || tspace <= 0) return FGB_ERR_ARG;
-  fgb_scripts *R = new fgb_scripts();
+  owner<fgb_scripts> own(new fgb_scripts(),fgb_scripts_free);
+  fgb_scripts *R = own.get();
   R->n = n;
   R->soff.assign(n+1,0);
   R->diffs.assign(n,0);
-  if (n == 0) { *out = R; return FGB_OK; }
+  if (n == 0) { *out = own.release(); return FGB_OK; }
 
   std::vector<TileJob> jobs;
   std::vector<AlnSeq> seqs(n);
@@ -174,8 +175,8 @@ extern "C" int fgb_compute_trace_pts(const fgb_genome *A, const fgb_genome *B, l
     { const int *f = fields + 9*i;
       const unsigned char *tr = pool + toff[i];
       const int ar = f[1], br = f[2], tlen = f[8];
-      if (ar < 0 || ar >= A->ncontig || br < 0 || br >= B->ncontig) { delete R; return FGB_ERR_ARG; }
-      if (f[0] && B->d_rseq == NULL) { delete R; return FGB_ERR_ARG; }
+      if (ar < 0 || ar >= A->ncontig || br < 0 || br >= B->ncontig) return FGB_ERR_ARG;
+      if (f[0] && B->d_rseq == NULL) return FGB_ERR_ARG;
       comp[i] = (unsigned char) (f[0] != 0);
       seqs[i].aw = A->woff[ar]; seqs[i].bw = B->woff[br];
       seqs[i].alen = (int) A->clen[ar]; seqs[i].blen = (int) B->clen[br];
@@ -189,7 +190,7 @@ extern "C" int fgb_compute_trace_pts(const fgb_genome *A, const fgb_genome *B, l
           const int d  = tlen >= 2 ? tr[2*t] : f[7];
           TileJob J;
           J.aln = (unsigned) i; J.a0 = a; J.m = ae - a; J.b0 = b; J.n = be - b;
-          if (J.m < 0 || J.n < 0 || ae > seqs[i].alen || be > seqs[i].blen) { delete R; return FGB_ERR_ARG; }
+          if (J.m < 0 || J.n < 0 || ae > seqs[i].alen || be > seqs[i].blen) return FGB_ERR_ARG;
           int del = J.m - J.n; if (del < 0) del = -del;
           J.dcap = d > del ? d - del : 0;
           J.out = (unsigned) slots; J.slab = slab;
@@ -200,32 +201,31 @@ extern "C" int fgb_compute_trace_pts(const fgb_genome *A, const fgb_genome *B, l
         }
     }
   first[n] = (long long) jobs.size();
-  if (slots >= 0xfffffff0ull || jobs.size() >= 0x7ffffff0ull) { delete R; return FGB_ERR_LIMIT; }
+  if (slots >= 0xfffffff0ull || jobs.size() >= 0x7ffffff0ull) return FGB_ERR_LIMIT;
 
   const int nj = (int) jobs.size();
   TileJob *d_jobs = NULL; AlnSeq *d_seqs = NULL; unsigned char *d_comp = NULL, *d_slab = NULL;
   int *d_script = NULL, *d_count = NULL, *d_td = NULL;
-  int rc = FGB_OK;
+  dev_scope S(st); S.own(d_jobs); S.own(d_seqs); S.own(d_comp); S.own(d_slab); S.own(d_script); S.own(d_count); S.own(d_td);
   std::vector<int> cnt(nj), td(nj), scr((size_t) slots + 1);
-#define TR_TRY(call) do { if ((call) != cudaSuccess) { rc = FGB_ERR_CUDA; goto done; } } while (0)
-  TR_TRY(fgb_dmalloc((void **) &d_jobs,sizeof(TileJob)*(size_t) nj,st));
-  TR_TRY(fgb_dmalloc((void **) &d_seqs,sizeof(AlnSeq)*(size_t) n,st));
-  TR_TRY(fgb_dmalloc((void **) &d_comp,(size_t) n,st));
-  TR_TRY(fgb_dmalloc((void **) &d_slab,(size_t) slab + 16,st));
-  TR_TRY(fgb_dmalloc((void **) &d_script,sizeof(int)*((size_t) slots + 1),st));
-  TR_TRY(fgb_dmalloc((void **) &d_count,sizeof(int)*(size_t) nj,st));
-  TR_TRY(fgb_dmalloc((void **) &d_td,sizeof(int)*(size_t) nj,st));
-  TR_TRY(cudaMemcpyAsync(d_jobs,jobs.data(),sizeof(TileJob)*(size_t) nj,cudaMemcpyHostToDevice,st));
-  TR_TRY(cudaMemcpyAsync(d_seqs,seqs.data(),sizeof(AlnSeq)*(size_t) n,cudaMemcpyHostToDevice,st));
-  TR_TRY(cudaMemcpyAsync(d_comp,comp.data(),(size_t) n,cudaMemcpyHostToDevice,st));
+  CUDA_TRY(fgb_dmalloc((void **) &d_jobs,sizeof(TileJob)*(size_t) nj,st));
+  CUDA_TRY(fgb_dmalloc((void **) &d_seqs,sizeof(AlnSeq)*(size_t) n,st));
+  CUDA_TRY(fgb_dmalloc((void **) &d_comp,(size_t) n,st));
+  CUDA_TRY(fgb_dmalloc((void **) &d_slab,(size_t) slab + 16,st));
+  CUDA_TRY(fgb_dmalloc((void **) &d_script,sizeof(int)*((size_t) slots + 1),st));
+  CUDA_TRY(fgb_dmalloc((void **) &d_count,sizeof(int)*(size_t) nj,st));
+  CUDA_TRY(fgb_dmalloc((void **) &d_td,sizeof(int)*(size_t) nj,st));
+  CUDA_TRY(cudaMemcpyAsync(d_jobs,jobs.data(),sizeof(TileJob)*(size_t) nj,cudaMemcpyHostToDevice,st));
+  CUDA_TRY(cudaMemcpyAsync(d_seqs,seqs.data(),sizeof(AlnSeq)*(size_t) n,cudaMemcpyHostToDevice,st));
+  CUDA_TRY(cudaMemcpyAsync(d_comp,comp.data(),(size_t) n,cudaMemcpyHostToDevice,st));
   trace_tiles_kernel<<<(nj + 127)/128,128,0,st>>>(d_jobs,nj,d_seqs,A->d_seq,B->d_seq,B->d_rseq,d_comp,d_slab,
                                                   d_script,d_count,d_td);
   fgb_count_launch(1);
-  TR_TRY(cudaGetLastError());
-  TR_TRY(cudaMemcpyAsync(cnt.data(),d_count,sizeof(int)*(size_t) nj,cudaMemcpyDeviceToHost,st));
-  TR_TRY(cudaMemcpyAsync(td.data(),d_td,sizeof(int)*(size_t) nj,cudaMemcpyDeviceToHost,st));
-  TR_TRY(cudaMemcpyAsync(scr.data(),d_script,sizeof(int)*(size_t) slots,cudaMemcpyDeviceToHost,st));
-  TR_TRY(cudaStreamSynchronize(st));
+  CUDA_TRY(cudaGetLastError());
+  CUDA_TRY(cudaMemcpyAsync(cnt.data(),d_count,sizeof(int)*(size_t) nj,cudaMemcpyDeviceToHost,st));
+  CUDA_TRY(cudaMemcpyAsync(td.data(),d_td,sizeof(int)*(size_t) nj,cudaMemcpyDeviceToHost,st));
+  CUDA_TRY(cudaMemcpyAsync(scr.data(),d_script,sizeof(int)*(size_t) slots,cudaMemcpyDeviceToHost,st));
+  CUDA_TRY(cudaStreamSynchronize(st));
   //  string the tiles of every alignment together
   R->script.reserve((size_t) slots);
   for (long long i = 0; i < n; i++)
@@ -240,11 +240,6 @@ extern "C" int fgb_compute_trace_pts(const fgb_genome *A, const fgb_genome *B, l
       R->diffs[i] = diffs;
     }
   R->soff[n] = (long long) R->script.size();
-done:
-#undef TR_TRY
-  fgb_dfree(d_jobs,st); fgb_dfree(d_seqs,st); fgb_dfree(d_comp,st); fgb_dfree(d_slab,st);
-  fgb_dfree(d_script,st); fgb_dfree(d_count,st); fgb_dfree(d_td,st);
-  if (rc) { delete R; return rc; }
-  *out = R;
+  *out = own.release();
   return FGB_OK;
 }

@@ -115,38 +115,6 @@ class DeviceGix:
         return cls(h)
 
     @classmethod
-    def build_range(cls, dgenome, plo, phi, stream=None):
-        L = load_library()
-        h = c_void_p()
-        L.fgb_gix_build_range.argtypes = [c_void_p, C.c_uint, C.c_uint, C.POINTER(c_void_p), c_void_p]
-        _check(L.fgb_gix_build_range(dgenome.h, plo, phi, C.byref(h), stream), "fgb_gix_build_range")
-        return cls(h)
-
-    @classmethod
-    def from_device(cls, dev_ptr, n, post_bytes, cont_bytes, ncontig, stream=None):
-        L = load_library()
-        h = c_void_p()
-        L.fgb_gix_from_device.argtypes = [c_void_p, c_ll, c_int, c_int, c_int, C.POINTER(c_void_p), c_void_p]
-        _check(L.fgb_gix_from_device(c_void_p(dev_ptr), n, post_bytes, cont_bytes, ncontig, C.byref(h), stream),
-               "fgb_gix_from_device")
-        return cls(h)
-
-    def copy_table_to(self, dev_ptr, stream=None):
-        L = load_library()
-        L.fgb_gix_copy_table.argtypes = [c_void_p, c_void_p, c_void_p]
-        _check(L.fgb_gix_copy_table(self.h, c_void_p(dev_ptr), stream), "fgb_gix_copy_table")
-
-    @classmethod
-    def upload(cls, tab, post_bytes, cont_bytes, ncontig, stream=None):
-        L = load_library()
-        h = c_void_p()
-        tab = np.ascontiguousarray(tab, dtype=np.uint64).reshape(-1, 2)
-        L.fgb_gix_upload.argtypes = [c_void_p, c_ll, c_int, c_int, c_int, C.POINTER(c_void_p), c_void_p]
-        _check(L.fgb_gix_upload(_ptr(tab), tab.shape[0], post_bytes, cont_bytes, ncontig,
-                                C.byref(h), stream), "fgb_gix_upload")
-        return cls(h)
-
-    @classmethod
     def import_ktab(cls, gixfile, stream=None):
         L = load_library()
         h = c_void_p()
@@ -460,22 +428,6 @@ def align_resident(dA, dB, freqA, stream=None, **kw):
     return _alns_out(h), st.asdict()
 
 
-def align_tables(dA, dB, xA, xB, freqA, stream=None, **kw):
-    """merge + seed sort + extension + filter from prebuilt tables"""
-    p = dict(DEFAULTS)
-    p.update(kw)
-    L = load_library()
-    h = c_void_p()
-    st = RunStats()
-    f = np.ascontiguousarray(freqA, dtype=np.float32)
-    L.fgb_align_tables.argtypes = [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int,
-                                   C.c_double, C.POINTER(c_void_p), C.POINTER(RunStats), c_void_p]
-    _check(L.fgb_align_tables(dA.h, dB.h, xA.h, xB.h, _ptr(f), p["freq"], p["chain_break"], p["chain_min"],
-                              p["align_min"], float(p["align_rate"]), C.byref(h), C.byref(st), stream),
-           "fgb_align_tables")
-    return _alns_out(h), st.asdict()
-
-
 def fastga_self(g, stream=None, **kw):
     """SELF mode, `FastGA A` with one source (formats.Genome) -> (Alignments, stats)"""
     p = dict(DEFAULTS)
@@ -573,16 +525,6 @@ def kmers_scan(dgenome, mask, fwd_only, stream=None):
     L.fgb_kmers_scan.argtypes = [c_void_p, c_void_p, c_int, C.POINTER(c_void_p), C.POINTER(c_ll), c_void_p]
     _check(L.fgb_kmers_scan(dgenome.h, _ptr(m), int(fwd_only), C.byref(ptr), C.byref(n), stream), "fgb_kmers_scan")
     return ptr.value, n.value
-
-
-def records_group_by_top_byte(src_ptr, n, dst_ptr, stream=None):
-    """groups n records by the first four bases of the k-mer into dst; returns bounds[257]"""
-    L = load_library()
-    bounds = np.zeros(257, dtype=np.int64)
-    L.fgb_records_group_by_top_byte.argtypes = [c_void_p, c_ll, c_void_p, c_void_p, c_void_p]
-    _check(L.fgb_records_group_by_top_byte(c_void_p(src_ptr), n, c_void_p(dst_ptr), _ptr(bounds), stream),
-           "fgb_records_group_by_top_byte")
-    return bounds
 
 
 def records_group_by_owner(src_ptr, n, owner256, world, dst_ptr, stream=None):

@@ -1,19 +1,6 @@
-"""Multi-GPU plumbing of the path: contig sharding (no data-path collective) and the gather of the
-per-rank alignment record streams (the only collective, SURVEY 8e)."""
+"""Multi-GPU plumbing of the path: k-mer-space sharding (two all-to-alls of 16-byte records) and the
+gather of the per-rank alignment record streams on rank 0."""
 import numpy as np
-
-
-def shard_contigs(lengths, rank, world):
-    """Greedy length balance of genome-1 contigs over ranks, longest first (the reference balances
-    its A-contig panels by bp the same way, FastGA.c:5067-5085).  Deterministic on every rank."""
-    order = np.argsort(-np.asarray(lengths, dtype=np.int64), kind="stable")
-    load = [0] * world
-    owner = np.zeros(len(lengths), dtype=np.int64)
-    for i in order:
-        r = int(np.argmin(load))
-        owner[int(i)] = r
-        load[r] += int(lengths[int(i)])
-    return [i for i in range(len(lengths)) if owner[i] == rank]
 
 
 def pack_alignments(alns, contig_map=None):
@@ -76,44 +63,6 @@ def merge_alignments(parts):
     order = np.lexsort((fields[:, 0], fields[:, 2], fields[:, 3], fields[:, 1]))
     return Alignments(fields[order], toff[order], pool if pool.size else np.zeros(1, np.uint8),
                       sum(p.nraw for p in parts))
-
-
-def build_table_cooperatively(dgenome, dist, device):
-    """Every rank scans the whole genome but keeps, sorts and indexes only the k-mers whose
-    12-base prefix falls in its 1/N slice of the prefix space; the sorted shares concatenate in
-    rank order into the complete table, exchanged with one NCCL all-gather over NVLink.  This is
-    the one real exchange step of the path when genome 2 is needed by every rank."""
-    import torch
-    from .lib import DeviceGix
-    rank, world = dist.get_rank(), dist.get_world_size()
-    if world == 1:
-        return DeviceGix.build(dgenome)
-    plo, phi = (rank << 24) // world, ((rank + 1) << 24) // world
-    share = DeviceGix.build_range(dgenome, plo, phi)
-    n_local = share.n
-    sizes = [torch.zeros(1, dtype=torch.int64, device=device) for _ in range(world)]
-    dist.all_gather(sizes, torch.tensor([n_local], dtype=torch.int64, device=device))
-    sizes = [int(s.item()) for s in sizes]
-    mx = max(sizes)
-    local = torch.empty(mx * 16, dtype=torch.uint8, device=device)
-    share.copy_table_to(local.data_ptr())
-    pb, cb = share.post_bytes, share.cont_bytes
-    share.close()
-    gathered = torch.empty(world * mx * 16, dtype=torch.uint8, device=device)
-    dist.all_gather_into_tensor(gathered, local)
-    total = sum(sizes)
-    if all(s == mx for s in sizes):
-        full = gathered
-    else:
-        full = torch.empty(total * 16, dtype=torch.uint8, device=device)
-        o = 0
-        for r, s in enumerate(sizes):
-            full[o:o + s * 16] = gathered[r * mx * 16: r * mx * 16 + s * 16]
-            o += s * 16
-    torch.cuda.synchronize()
-    gx = DeviceGix.from_device(full.data_ptr(), total, pb, cb, dgenome.genome.ncontig)
-    del gathered, full, local
-    return gx
 
 
 # ---------------------------------------------------------------------------------------------

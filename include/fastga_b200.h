@@ -82,11 +82,6 @@ int fgb_align_resident(const fgb_genome *A, const fgb_genome *B, const float *fr
                        int freq, int chain_break, int chain_min, int align_min, double align_rate,
                        fgb_alns **out, fgb_run_stats *stats, void *stream);
 
-/* Same from prebuilt tables (x2 possibly assembled from per-rank shares). */
-int fgb_align_tables(const fgb_genome *A, const fgb_genome *B, const fgb_gix *x1, const fgb_gix *x2,
-                     const float *freqA, int freq, int chain_break, int chain_min, int align_min,
-                     double align_rate, fgb_alns **out, fgb_run_stats *stats, void *stream);
-
 /* ---- genome (GDB.h:28-72; Get_Contig / Get_Contig_Piece GDB.c:1739,1841; Complement_Seq) ---- */
 int  fgb_genome_create(const unsigned char *bps, long long bps_bytes, int ncontig,
                        const long long *clen, const long long *boff, int want_revcomp,
@@ -104,14 +99,6 @@ int  fgb_gix_build(const fgb_genome *g, fgb_gix **out, void *stream);
 /* forward-strand entries only: enough for the genome that supplies the adaptamers (its reverse
    entries never seed, FastGA.c:921-928); fgb_seeds_find compacts a both-strand table itself */
 int  fgb_gix_build_forward(const fgb_genome *g, fgb_gix **out, void *stream);
-/* one rank's share (12-base prefix in [plo,phi)) of a cooperatively built table, and the pieces
-   to assemble the shares gathered over NCCL (fastga_b200/shard.py) */
-int  fgb_gix_build_range(const fgb_genome *g, unsigned plo, unsigned phi, fgb_gix **out, void *stream);
-int  fgb_gix_copy_table(const fgb_gix *x, void *d_dst, void *stream);
-int  fgb_gix_from_device(const void *d_tab, long long n, int post_bytes, int cont_bytes, int ncontig,
-                         fgb_gix **out, void *stream);
-int  fgb_gix_upload(const void *tab, long long n, int post_bytes, int cont_bytes, int ncontig,
-                    fgb_gix **out, void *stream);
 /* entries = concatenated .ktab parts, index = the stub's cumulative 2^24 table (libfastk.c:815-840) */
 int  fgb_gix_import_ktab(const unsigned char *entries, long long n, int post_bytes, int cont_bytes,
                          const long long *index, int ncontig, fgb_gix **out, void *stream);
@@ -212,10 +199,8 @@ void fgb_device_free(void *p);
 /* unsorted k-mer records of the contigs with mask[c] != 0; fwd_only drops reverse-strand entries */
 int  fgb_kmers_scan(const fgb_genome *g, const unsigned char *mask, int fwd_only,
                     void **d_recs, long long *n, void *stream);
-/* d_out[bounds257[b] .. bounds257[b+1]) = the records whose top k-mer byte is b (d_recs is scratch) */
-int  fgb_records_group_by_top_byte(void *d_recs, long long n, void *d_out, long long *bounds257,
-                                   void *stream);
-/* the same by destination only: owner256[b] = rank owning top byte b; d_out[bounds[w] .. bounds[w+1]) */
+/* records grouped by destination: owner256[b] = rank owning top k-mer byte b; d_out[bounds[w] .. bounds[w+1])
+   = the records of rank w */
 int  fgb_records_group_by_owner(const void *d_recs, long long n, const int *owner256, int world,
                                 void *d_out, long long *bounds, void *stream);
 /* sorted + indexed table over records whose 12-base prefix lies in [plo,phi) (one rank's slice) */

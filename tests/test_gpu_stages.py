@@ -80,8 +80,20 @@ def test_gix_build_with_heavy_repeats_matches_oracle():
     assert np.array_equal(pstart, wstart)
 
 
+def _share_from_records(g, full, lo, hi, seed):
+    """one rank's slice of a k-mer-space sharded table the way the sharded path builds it
+    (fgb_gix_from_records): the rows of the full table whose 12-base prefix lies in [lo, hi), in a
+    seeded random order on the device"""
+    import torch
+    rows = full[((full[:, 1] >> np.uint64(40)) >= lo) & ((full[:, 1] >> np.uint64(40)) < hi)]
+    rows = rows[np.random.default_rng(seed).permutation(len(rows))]
+    recs = torch.from_numpy(rows.view(np.int64).copy()).cuda()
+    pb, cb = formats.gix_bytes(g)
+    return lib.gix_from_records(recs.data_ptr() if len(rows) else 0, len(rows), lo, hi, False, pb, cb, g.ncontig)
+
+
 @pytest.mark.parametrize("target", ["8", "1"])
-def test_gix_build_with_more_than_65536_bins_is_the_same_table(small_pair, target):
+def test_gix_with_more_than_65536_bins_is_the_same_table_whole_and_from_records(small_pair, target):
     """tables beyond ~100 M records are partitioned into more than 2^16 prefix bins (a third, narrower
     digit pass) so that a bin still fits a CTA's shared memory; FGB_KSORT_BIN_TARGET forces that regime
     on a small table (2^19 .. 2^22 bins here), whole table and shares alike"""
@@ -92,24 +104,24 @@ def test_gix_build_with_more_than_65536_bins_is_the_same_table(small_pair, targe
     os.environ["FGB_KSORT_BIN_TARGET"] = target
     try:
         tab2, pstart2, _ = lib.DeviceGix.build(dg).download()
-        parts = [lib.DeviceGix.build_range(dg, lo, hi).download()[0]
-                 for lo, hi in ((0, (1 << 23) + 5), ((1 << 23) + 5, 1 << 24))]
+        parts = [_share_from_records(g, full, lo, hi, k).download()[0]
+                 for k, (lo, hi) in enumerate(((0, (1 << 23) + 5), ((1 << 23) + 5, 1 << 24)))]
     finally:
         del os.environ["FGB_KSORT_BIN_TARGET"]
     assert np.array_equal(tab2, full) and np.array_equal(pstart2, pstart)
     assert np.array_equal(np.concatenate(parts), full)
 
 
-def test_gix_shares_of_the_prefix_space_concatenate_to_the_full_table(small_pair):
-    """one rank's share of a cooperatively built table (fgb_gix_build_range) is binned relative to
+def test_gix_slices_from_records_concatenate_to_the_full_table(small_pair):
+    """one rank's slice of a k-mer-space sharded table (fgb_gix_from_records) is binned relative to
     its own prefix range; uneven shares must concatenate to exactly the single-GPU table"""
     g = small_pair[1]
     dg = lib.DeviceGenome(g)
     full, _, _ = lib.DeviceGix.build(dg).download()
     cuts = [0, 1 << 21, (1 << 23) + 12345, (3 << 22) + 7, 1 << 24]
     parts = []
-    for lo, hi in zip(cuts[:-1], cuts[1:]):
-        sh = lib.DeviceGix.build_range(dg, lo, hi)
+    for k, (lo, hi) in enumerate(zip(cuts[:-1], cuts[1:])):
+        sh = _share_from_records(g, full, lo, hi, k)
         tab = sh.download()[0]
         assert len(tab) == sh.n
         if sh.n:

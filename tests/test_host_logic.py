@@ -76,16 +76,6 @@ def test_ktab_lcp_and_canonical_form():
     assert list(lcp) == [0, 40, 39, 0]
 
 
-def test_shard_contigs_partition():
-    lens = [50, 10, 40, 30, 20, 60, 5]
-    for world in (1, 2, 3, 8):
-        parts = [shard.shard_contigs(lens, r, world) for r in range(world)]
-        flat = sorted(i for p in parts for i in p)
-        assert flat == list(range(len(lens)))
-        loads = [sum(lens[i] for i in p) for p in parts]
-        assert max(loads) - min(loads) <= max(lens)
-
-
 def test_kmer_space_ownership_covers_everything_once():
     """the sharded path's two ownership maps: k-mer prefix ranges (by the first four bases) tile the
     prefix space, contigs are spread by length"""
